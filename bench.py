@@ -2,6 +2,7 @@
 """bench.py - PnP-ADMM MRF reconstruction + dictionary matching on B200 (contract: the task's bench section).
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--mask spiral|epi] [--slices 120] [--iters 100]
+                    [--dump-outputs DIR]
 
 Metric (BASELINE.json): ADMM slice-iterations/s on 224 x 224 x 10 slices, whole job over all N GPUs.
 Workload (north star, BASELINE configs[3]): the 120-slice job (8 synthetic volunteers x 15 slices, QMaps rendered through the
@@ -35,6 +36,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True   # the benchmark may run from a read-only tree and leaves nothing in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for _p in (ROOT, os.path.join(ROOT, "qmri-pnp-recon-poc_b200")):
     if _p not in sys.path:
@@ -486,6 +488,8 @@ def run_ours(args, rank, world, local_rank):
     if clocks is not None:
         clocks["how"] = f"NVML queries every {args.clock_period} s during the timed pass `value` is taken from"
     value = args.slices * iters * args.steps / (ms_dev * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, args.slices, g0, sess, Xout, qmap_d, pd_d, dist, rank)
     # share of matching inside the step (same data, same stream)
     ms_match, _ = timed(match_resident, 2, 1, label="matching only", do_flush=False)
 
@@ -643,6 +647,39 @@ def run_ours(args, rank, world, local_rank):
         dist.destroy_process_group()
 
 
+DUMP_PIXELS = 1 << 19   # 96 B per pixel (x: C complex channels, qmap: T1 and T2, pd: complex) -> 48 MiB of files at most
+
+
+def dump_outputs(path, slices, g0, sess, x_host, qmap_d, pd_d, dist, rank):
+    """What the timed step hands its caller, taken from its last step: x = PnP_ADMM(y, param) and out.qmap / out.pd of
+    mrf_dtm_cpu, at the same pixels of the job - all of them when the job has at most DUMP_PIXELS, else a sorted sample drawn
+    with a fixed seed (independent of the number of ranks).  Written as float32 to path/x.npy [P x C x 2] (re, im of every
+    channel), path/qmap.npy [P x 2] (T1, T2) and path/pd.npy [P x 2] (re, im); pixel g is slice g // (N M), column-major
+    pixel g % (N M) of that slice."""
+    import torch
+    S = x_host.shape[3]
+    total = slices * HW
+    pick = np.arange(total) if total <= DUMP_PIXELS else np.sort(np.random.default_rng(0).choice(total, DUMP_PIXELS, replace=False))
+    mine = (pick >= g0 * HW) & (pick < (g0 + S) * HW)
+    s, p = np.divmod(pick[mine] - g0 * HW, HW)
+    sess.download(x_host)
+    x = x_host.reshape((HW, C_CH, S), order="F")[p, :, s]                       # P_mine x C complex
+    rows = np.zeros((pick.size, 2 * C_CH + 4), np.float32)
+    rows[mine, :2 * C_CH] = np.stack([x.real, x.imag], axis=2).reshape(-1, 2 * C_CH)
+    rows[mine, 2 * C_CH:2 * C_CH + 2] = qmap_d.view(S, 2, HW).cpu().numpy()[s, :, p]   # per slice: npix x 2 column-major
+    rows[mine, 2 * C_CH + 2:] = pd_d.view(S, HW, 2).cpu().numpy()[s, p]              # per slice: npix complex interleaved
+    if dist is not None:   # every rank fills the rows of its own slices
+        t = torch.from_numpy(rows).cuda()
+        dist.all_reduce(t, op=dist.ReduceOp.SUM)
+        rows = t.cpu().numpy()
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+        np.save(os.path.join(path, "x.npy"), rows[:, :2 * C_CH].reshape(-1, C_CH, 2))
+        np.save(os.path.join(path, "qmap.npy"), rows[:, 2 * C_CH:2 * C_CH + 2])
+        np.save(os.path.join(path, "pd.npy"), rows[:, 2 * C_CH + 2:])
+        sys.stderr.write(f"[bench] outputs of the last timed step ({pick.size} of {total} pixels) written to {path}\n")
+
+
 def run_extras(args, q, ctx, net, F, d, dct, Yp, X0p, timed, log, rank, world, dist, stream, peaks):
     """Short legs for the other BASELINE configs (reported beside the headline, never part of `value`)."""
     import torch
@@ -729,7 +766,11 @@ def main():
     ap.add_argument("--k1-idle", type=float, default=4.0, help="idle seconds before the x-update-alone roofline leg (lets the power cap release)")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write x, qmap and pd of the last timed step to DIR/<name>.npy (float32; "
+                                                          f"a fixed, seeded sample of {DUMP_PIXELS} pixels when the job has more)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # launched by hand without torchrun: start one rank per GPU the way the driver does
         port = 29500 + os.getpid() % 2000
