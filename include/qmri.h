@@ -84,7 +84,8 @@ const char* qmri_last_error(void);
  *   setup_subsampling_epi(N,M,percentage,V)  main_files/subsampling_patterns/setup_subsampling_epi.m:1-37
  * and the closures F.forward / F.adjoint of main_recon_tsmis_FFT.m:228-229.
  * V is L x C column-major, real (the reference passes real(dict.V)).
- * Scope of this build: N == M == 224.  V == eye(C) (the BASELINE configuration) takes the diagonal data-consistency
+ * Scope of this build: N == M == 224 or N == M == 256 (other sizes: QMRI_EUNSUPPORTED).  At 256 the x-update runs on the
+ * streaming kernels at every batch size (QMRI_K1_KERNEL=cluster is refused; QMRI_K1_STATE=real runs the complex loop).  V == eye(C) (the BASELINE configuration) takes the diagonal data-consistency
  * path; any other real L x C V (C <= 16) takes the exact per-location block solve on the union of the L masks
  * (SURVEY.md 8f-2; the union is processed in parts of <= 3400 k-space locations, e.g. 4 parts for 200 spiral frames).
  */

@@ -140,24 +140,26 @@ static void emulate(int mode, int C, int S, const optab::K1Tables& t, const floa
     }
 }
 
-// Streaming kernels (xupdate_stream.cu): forward kernel per slab group (G CTAs per image, 224 threads each), solve kernel,
+// Streaming kernels (xupdate_stream.cu): forward kernel per slab group (G CTAs per image, N threads each), solve kernel,
 // adjoint kernel - same control flow, thread by thread.
+template <int N>
 static void emulate_stream(int mode, int C, int S, const optab::K1Tables& t, const float* in_re, const float* in_im,
                            const float* v, const float* y, float rho, float* out_re, float* out_im, float* y_out,
                            float* minmax) {
-    constexpr int MC = HC_STREAM, THREADS = 16 * MC, SLABS = NF / MC, G = 4, SPC = SLABS / G;
+    constexpr int MC = Side<N>::R, CS = Side<N>::CS, NP = Side<N>::NP, OVF_STRIDE = Side<N>::OVF_STRIDE;
+    constexpr int THREADS = 16 * MC, SLABS = N / MC, G = 4, SPC = SLABS / G;
     const float2* tw2 = reinterpret_cast<const float2*>(t.tw2.data());
     const float2* tw448 = reinterpret_cast<const float2*>(t.tw448.data());
-    const size_t plane = (size_t)NF * NF;
-    const float inv_n = 1.0f / (float)NF;
+    const size_t plane = (size_t)N * N;
+    const float inv_n = 1.0f / (float)N;
     for (int s = 0; s < S; ++s) {
         float lmin = INFINITY, lmax = -INFINITY;
         for (int c = 0; c < C; ++c) {
             const int f0 = t.frame_ptr[c], ns = t.frame_ptr[c + 1] - f0;
             const size_t img = ((size_t)(s * C + c)) * plane;
             const uint32_t* ent = t.ent.data() + f0;
-            const uint32_t* itA = t.itA.data() + (size_t)c * NF;
-            const uint32_t* itB = t.itB.data() + (size_t)c * NF;
+            const uint32_t* itA = t.itA.data() + (size_t)c * N;
+            const uint32_t* itB = t.itB.data() + (size_t)c * N;
             std::vector<float2> regs((size_t)THREADS * 16);
             auto A = [&](int tid) -> float2(&)[16] { return *reinterpret_cast<float2(*)[16]>(&regs[(size_t)tid * 16]); };
             std::vector<float2> cvec((size_t)t.ns_max + 1, float2{0, 0});
@@ -175,9 +177,9 @@ static void emulate_stream(int mode, int C, int S, const optab::K1Tables& t, con
                         const int m0 = (g * SPC + sl) * MC;
                         for (int tid = 0; tid < THREADS; ++tid) {
                             const int l16 = tid & 15, col = tid >> 4;
-                            const size_t gi = img + (size_t)(m0 + col) * NF + l16;
+                            const size_t gi = img + (size_t)(m0 + col) * N + l16;
                             float2(&a)[16] = A(tid);
-                            for (int n1 = 0; n1 < 14; ++n1) {
+                            for (int n1 = 0; n1 < MC; ++n1) {
                                 float re = in_re[gi + 16 * n1], im = in_im ? in_im[gi + 16 * n1] : 0.f;
                                 if (mode == 0) {
                                     re = 2.f * v[gi + 16 * n1] - re;
@@ -185,15 +187,15 @@ static void emulate_stream(int mode, int C, int S, const optab::K1Tables& t, con
                                 }
                                 a[n1] = float2{re, im};
                             }
-                            fwd_s1_regs(a, l16, tw2);
+                            fwd_s1_regs<N>(a, l16, tw2);
                         }
-                        for (int tid = 0; tid < THREADS; ++tid) fft_s1_store(ws.data() + (tid >> 4) * CS, tid & 15, A(tid));
+                        for (int tid = 0; tid < THREADS; ++tid) fft_s1_store<N>(ws.data() + (tid >> 4) * CS, tid & 15, A(tid));
                         for (int tid = 0; tid < THREADS; ++tid)
-                            if ((tid & 15) < 14) fft_s2_load(ws.data() + (tid >> 4) * CS, tid & 15, A(tid));
+                            if ((tid & 15) < MC) fft_s2_load(ws.data() + (tid >> 4) * CS, tid & 15, A(tid));
                         for (int tid = 0; tid < THREADS; ++tid)
-                            if ((tid & 15) < 14) fft_s2_store<false>(ws.data() + (tid >> 4) * CS, tid & 15, A(tid));
+                            if ((tid & 15) < MC) fft_s2_store<false, N>(ws.data() + (tid >> 4) * CS, tid & 15, A(tid));
                         for (int tid = 0; tid < THREADS; ++tid)
-                            p3_item(ws.data(), (int)(itA[tid] & 0xffu), ent + (itA[tid] >> 16), (int)((itA[tid] >> 8) & 0xffu), tw448, m0, pc.data());
+                            p3_item<N>(ws.data(), (int)(itA[tid] & 0xffu), ent + (itA[tid] >> 16), (int)((itA[tid] >> 8) & 0xffu), tw448, m0, pc.data());
                     }
                 }
                 for (int j = 0; j < ns; ++j) {  // solve kernel
@@ -223,28 +225,28 @@ static void emulate_stream(int mode, int C, int S, const optab::K1Tables& t, con
                     for (auto& e : ws) e = float2{NAN, NAN};  // rows without samples are never written: they must never be read either
                     for (int tid = 0; tid < THREADS; ++tid) {
                         const int k1row = (int)(itA[tid] & 0xffu), cnt = (int)((itA[tid] >> 8) & 0xffu), slot = (int)(itB[tid] & 0xffu);
-                        if (k1row != 255) {
-                            float2 SP[NP_STREAM], SM[NP_STREAM];
-                            p4_item_partial(SP, SM, ent + (itA[tid] >> 16), cnt, tw448, m0, cvec.data());
-                            if (slot == 0) p4_item_store(ws.data(), k1row, SP, SM);
-                            else p4_item_spill(ovf.data() + (size_t)(slot - 1) * OVF_STRIDE, SP, SM);
+                        if (cnt != 0) {
+                            float2 SP[NP], SM[NP];
+                            p4_item_partial<N>(SP, SM, ent + (itA[tid] >> 16), cnt, tw448, m0, cvec.data());
+                            if (slot == 0) p4_item_store<N>(ws.data(), k1row, SP, SM);
+                            else p4_item_spill<N>(ovf.data() + (size_t)(slot - 1) * OVF_STRIDE, SP, SM);
                         }
                     }
                     for (int tid = 0; tid < THREADS; ++tid) {
-                        const int k1row = (int)(itA[tid] & 0xffu), slot = (int)(itB[tid] & 0xffu);
+                        const int k1row = (int)(itA[tid] & 0xffu), cnt = (int)((itA[tid] >> 8) & 0xffu), slot = (int)(itB[tid] & 0xffu);
                         const int novf = (int)((itB[tid] >> 8) & 0xffu), ovf0 = (int)((itB[tid] >> 16) & 0xffu);
-                        if (k1row != 255 && slot == 0 && novf) p4_row_add_overflow(ws.data(), k1row, ovf.data() + (size_t)ovf0 * OVF_STRIDE, novf);
+                        if (cnt != 0 && slot == 0 && novf) p4_row_add_overflow<N>(ws.data(), k1row, ovf.data() + (size_t)ovf0 * OVF_STRIDE, novf);
                     }
                     for (int tid = 0; tid < THREADS; ++tid)
-                        if ((tid & 15) < 14) inv_s1_load(ws.data() + (tid >> 4) * CS, tid & 15, tw2, t.rowmask[(size_t)c * 16 + (tid & 15)], A(tid));
+                        if ((tid & 15) < MC) inv_s1_load<N>(ws.data() + (tid >> 4) * CS, tid & 15, tw2, t.rowmask[(size_t)c * 16 + (tid & 15)], A(tid));
                     for (int tid = 0; tid < THREADS; ++tid)
-                        if ((tid & 15) < 14) inv_s1_store(ws.data() + (tid >> 4) * CS, tid & 15, A(tid));
+                        if ((tid & 15) < MC) inv_s1_store(ws.data() + (tid >> 4) * CS, tid & 15, A(tid));
                     for (int tid = 0; tid < THREADS; ++tid) {
                         const int l16 = tid & 15, col = tid >> 4;
-                        const size_t gi = img + (size_t)(m0 + col) * NF + l16;
+                        const size_t gi = img + (size_t)(m0 + col) * N + l16;
                         float2(&a)[16] = A(tid);
-                        inv_s2_regs(ws.data() + col * CS, l16, a);
-                        for (int d = 0; d < 14; ++d) {
+                        inv_s2_regs<N>(ws.data() + col * CS, l16, a);
+                        for (int d = 0; d < MC; ++d) {
                             float ore, oim;
                             if (mode == 0) {
                                 ore = v[gi + 16 * d] + a[d].x;
@@ -338,7 +340,7 @@ static void emulate_real(int op, int C, int S, const optab::K1Tables& t, const f
                     for (auto& e : ws) e = float2{NAN, NAN};  // rows outside the symmetric row mask are never written nor read
                     for (int tid = 0; tid < THREADS; ++tid) {
                         const int k1row = (int)(itA[tid] & 0xffu), cnt = (int)((itA[tid] >> 8) & 0xffu), slot = (int)(itB[tid] & 0xffu);
-                        if (k1row == 255) continue;
+                        if (cnt == 0) continue;
                         for (int h = 0; h < 2; ++h) {
                             float2 SP[NP_STREAM], SM[NP_STREAM];
                             p4r_item_partial(SP, SM, ent + (itA[tid] >> 16), cnt, tw448, m0 + 14 * h, cvec.data());
@@ -347,9 +349,9 @@ static void emulate_real(int op, int C, int S, const optab::K1Tables& t, const f
                         }
                     }
                     for (int tid = 0; tid < THREADS; ++tid) {
-                        const int k1row = (int)(itA[tid] & 0xffu), slot = (int)(itB[tid] & 0xffu);
+                        const int k1row = (int)(itA[tid] & 0xffu), cnt = (int)((itA[tid] >> 8) & 0xffu), slot = (int)(itB[tid] & 0xffu);
                         const int novf = (int)((itB[tid] >> 8) & 0xffu), ovf0 = (int)((itB[tid] >> 16) & 0xffu);
-                        if (k1row != 255 && slot == 0 && novf)
+                        if (cnt != 0 && slot == 0 && novf)
                             for (int h = 0; h < 2; ++h)
                                 p4r_row_add_overflow(ws.data(), k1row, h, ovf.data() + ((size_t)ovf0 * 2 + h) * OVF_STRIDE, novf, 2 * OVF_STRIDE);
                     }
@@ -410,11 +412,45 @@ int k1emu_run(int mode, int mc, int pattern, double arg, int C, int S, const flo
     optab::build_k1_tables(NF, frames, t, env ? atoi(env) : 8);
     if (mc == 0) {  // streaming kernel
         if (!t.stream_ok) return -1;
-        emulate_stream(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax);
+        emulate_stream<NF>(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax);
         return t.nmeas;
     }
     if (mc == 56) emulate<56>(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax);
     else emulate<28>(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax);
+    return t.nmeas;
+}
+
+// The streaming kernels at image side n (224 or 256; N == M), same modes and arguments as k1emu_run.  Returns nmeas, -1 if the
+// mask does not fit the work-item tables, -2 for another side.
+int k1emu_run_n(int n, int mode, int pattern, double arg, int C, int S, const float* in_re, const float* in_im, const float* v,
+                const float* y, float rho, float* out_re, float* out_im, float* y_out, float* minmax) {
+    if (n != 224 && n != 256) return -2;
+    std::vector<std::vector<int32_t>> frames;
+    if (pattern == 0) optab::spiral_frames(n, (int)arg, C, frames);
+    else optab::epi_frames(n, n, arg, C, frames);
+    optab::K1Tables t;
+    const char* env = getenv("QMRI_K1_QMIN");
+    optab::build_k1_tables(n, frames, t, env ? atoi(env) : 8);
+    if (!t.stream_ok) return -1;
+    if (n == 224) emulate_stream<224>(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax);
+    else emulate_stream<256>(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax);
+    return t.nmeas;
+}
+
+// The streaming kernels' work-item tables (op_tables.h) at image side n for C frames of a mask: itA / itB [C][n], ent [nmeas],
+// rowmask [C][16] (each may be null).  Returns nmeas, -1 if the mask does not fit the tables.
+int k1emu_stream_tables(int n, int pattern, double arg, int C, uint32_t* itA, uint32_t* itB, uint32_t* ent, uint16_t* rowmask) {
+    std::vector<std::vector<int32_t>> frames;
+    if (pattern == 0) optab::spiral_frames(n, (int)arg, C, frames);
+    else optab::epi_frames(n, n, arg, C, frames);
+    optab::K1Tables t;
+    const char* env = getenv("QMRI_K1_QMIN");
+    optab::build_k1_tables(n, frames, t, env ? atoi(env) : 8);
+    if (!t.stream_ok) return -1;
+    if (itA) memcpy(itA, t.itA.data(), sizeof(uint32_t) * t.itA.size());
+    if (itB) memcpy(itB, t.itB.data(), sizeof(uint32_t) * t.itB.size());
+    if (ent) memcpy(ent, t.ent.data(), sizeof(uint32_t) * t.nmeas);
+    if (rowmask) memcpy(rowmask, t.rowmask.data(), sizeof(uint16_t) * t.rowmask.size());
     return t.nmeas;
 }
 

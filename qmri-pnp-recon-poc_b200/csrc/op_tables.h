@@ -76,24 +76,24 @@ struct K1Tables {
     std::vector<uint16_t> samp;       // [nmeas]
     std::vector<uint32_t> p4tab;      // [C][8][p4_len] flat work lists of the sparse inverse pass (see build_k1_tables)
     int p4_len = 0;
-    std::vector<float> tw;            // [224][2]
+    std::vector<float> tw;            // [N][2]
     // streaming kernel (xupdate_stream.cu): work items of the sparse m-direction sums (see build_stream_tables)
-    bool stream_ok = false;           // false: some frame needs more than 224 items / too many overflow partials
-    std::vector<uint32_t> itA;        // [C][N] k1 | cnt << 8 | start << 16   (k1 == 255: thread has no item)
+    bool stream_ok = false;           // false: some frame needs more than N items / too many overflow partials
+    std::vector<uint32_t> itA;        // [C][N] k1 | cnt << 8 | start << 16   (cnt == 0: thread has no item; the word is then 255)
     std::vector<uint32_t> itB;        // [C][N] slot | novf << 8 | ovf0 << 16
     std::vector<uint32_t> ent;        // [nmeas] j | k2 << 16, frame-major, grouped by item
-    std::vector<uint16_t> rowmask;    // [C][16] bit a of entry b: row 14 a + b holds samples (inverse FFT stage 1 skips empty rows)
+    std::vector<uint16_t> rowmask;    // [C][16] bit a of entry b: row R a + b (R = N / 16) holds samples (inverse FFT stage 1 skips empty rows)
     int n_ovf = 0;                    // largest number of overflow partials in one frame
     int max_row = 0;                  // largest number of samples in one row of one frame
     // real-image variant of the streaming kernels (xupdate_real.cu): the same work-item tables over FOLDED rows.  For a real image
     // the n-direction transform is Hermitian, T(N - k1, m) = conj T(k1, m), so a sample (k1 > N/2, k2) is carried by row N - k1 as
     // (N - k2) mod N with its value conjugated: entries j | k2' << 16 | conj << 31, rows 0 .. N/2 only.
-    bool real_ok = false;
+    bool real_ok = false;             // N == 224 only
     std::vector<uint32_t> r_itA, r_itB, r_ent;
     std::vector<uint16_t> r_rowmask;  // [C][16] like rowmask, symmetric: row k and row N - k are set together
     int r_n_ovf = 0;
     std::vector<float> tw2;           // [16][16][2]  e^{-2 pi i (i j) / N}
-    std::vector<float> tw448;         // [2N][2]      e^{-2 pi i t / (2N)}
+    std::vector<float> tw448;         // [2N][2]      e^{-2 pi i t / (2N)} (448 entries at N = 224, 512 at N = 256)
 };
 
 constexpr int K1_PHASES = 8;          // row phases of the sparse inverse pass = THREADS / MC of the kernel
@@ -106,7 +106,9 @@ static inline uint32_t p4_entry(int k2, int k1, int j, bool last) {
 constexpr int STREAM_QMAX = 64;      // == k1::QMAX_STREAM
 constexpr int STREAM_OVF_MAX = 96;   // == k1::OVF_MAX_STREAM
 
-// Work items of the streaming kernel.  The samples of a k-space row k1 are cut into chunks of at most Q samples (Q = the
+// Work items of the streaming kernel (N = 224 or 256 threads, one per k-space row).  Every item carries at least one sample, so
+// cnt == 0 marks a thread without an item (k1 takes all 8 bits: row 255 is a real row at N = 256).
+// The samples of a k-space row k1 are cut into chunks of at most Q samples (Q = the
 // smallest value for which the frame needs no more than N items, so a thread never carries more than one); the row's first
 // chunk is its PRIMARY item (it writes the row in the inverse pass), the others are OVERFLOW items whose partial sums go
 // through numbered shared-memory slots and are added by the primary in slot order (deterministic, no atomics).  Rows
@@ -177,7 +179,7 @@ static inline bool stream_items_for_frame(int N, const std::vector<std::vector<u
 }
 
 static inline void build_stream_tables(int N, const std::vector<std::vector<int32_t>>& frames, K1Tables& t, int q_min = 1) {
-    t.stream_ok = (N % 16 == 0) && N <= 254;
+    t.stream_ok = N == 224 || N == 256;  // the sides the streaming kernels are instantiated for
     t.itA.assign((size_t)t.C * N, 255u);
     t.itB.assign((size_t)t.C * N, 0u);
     t.ent.assign(std::max(t.nmeas, 1), 0);
@@ -202,7 +204,7 @@ static inline void build_stream_tables(int N, const std::vector<std::vector<int3
         }
         for (int k = 0; k < N; ++k) {
             t.max_row = std::max(t.max_row, (int)rows[k].size());
-            if (!rows[k].empty() && N == 224) t.rowmask[(size_t)c * 16 + k % 14] |= (uint16_t)(1u << (k / 14));
+            if (!rows[k].empty()) t.rowmask[(size_t)c * 16 + k % (N / 16)] |= (uint16_t)(1u << (k / (N / 16)));
             if (!folded[k].empty() && N == 224) {
                 const int kn = (N - k) % N;
                 t.r_rowmask[(size_t)c * 16 + k % 14] |= (uint16_t)(1u << (k / 14));

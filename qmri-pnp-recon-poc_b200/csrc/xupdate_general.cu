@@ -15,7 +15,6 @@
 namespace {
 
 constexpr int CMAX = 16;
-constexpr float INV_N = 1.0f / 224.0f;  // unitary scaling 1/sqrt(N*M), once per transform direction
 
 __device__ __forceinline__ float2 zhat(const GeneralMix& m, int s, int c, int u) {
     const float2* p = m.part + (((size_t)s * m.C + c) * m.G) * (size_t)m.nU + u;
@@ -25,7 +24,7 @@ __device__ __forceinline__ float2 zhat(const GeneralMix& m, int s, int c, int u)
         sx += t.x;
         sy += t.y;
     }
-    return make_float2(sx * INV_N, sy * INV_N);
+    return make_float2(sx * m.inv_n, sy * m.inv_n);
 }
 
 __global__ void __launch_bounds__(128) mix_forward_kernel(GeneralMix m) {
@@ -60,7 +59,7 @@ __global__ void __launch_bounds__(128) mix_adjoint_kernel(GeneralMix m) {
     }
 #pragma unroll
     for (int c = 0; c < CMAX; ++c)
-        if (c < m.C) m.cbuf[((size_t)s * m.C + c) * m.nU + u] = make_float2(tx[c] * INV_N, ty[c] * INV_N);
+        if (c < m.C) m.cbuf[((size_t)s * m.C + c) * m.nU + u] = make_float2(tx[c] * m.inv_n, ty[c] * m.inv_n);
 }
 
 __global__ void __launch_bounds__(128) mix_solve_kernel(GeneralMix m) {
@@ -107,7 +106,7 @@ __global__ void __launch_bounds__(128) mix_solve_kernel(GeneralMix m) {
                     dx = fmaf(w, tx[c], dx);
                     dy = fmaf(w, ty[c], dy);
                 }
-            m.cbuf[((size_t)s * m.C + r) * m.nU + u] = make_float2(dx * INV_N, dy * INV_N);  // pre-scaled for the inverse transform
+            m.cbuf[((size_t)s * m.C + r) * m.nU + u] = make_float2(dx * m.inv_n, dy * m.inv_n);  // pre-scaled for the inverse transform
         }
 }
 

@@ -23,16 +23,16 @@ struct K1Params {
     float2* y_out;        // FORWARD: [S][nmeas]
     int* minmax;          // optional [S][2] ordered-int min / max of out_re
     // per-operator tables (device)
-    const float2* tw;        // [224] e^{-2 pi i t / 224}
+    const float2* tw;        // [N] e^{-2 pi i t / N}
     const int* frame_ptr;    // [C+1]
-    const uint16_t* samp;    // [nmeas] k1 | k2 << 8, frame-major, ascending k = k1 + 224 k2
+    const uint16_t* samp;    // [nmeas] k1 | k2 << 8, frame-major, ascending k = k1 + N k2
     const uint32_t* p4tab;   // [C][8][p4_len] flat work lists of the sparse inverse pass (op_tables.h)
     int p4_len;
     // streaming kernel tables (xupdate_stream.cu; op_tables.h)
-    const float2* tw2;       // [16][16] e^{-2 pi i (i j) / 224}
-    const float2* tw448;     // [448] e^{-2 pi i t / 448}
-    const uint32_t* itA;     // [C][224] work item of thread tid: k1 | cnt << 8 | start << 16
-    const uint32_t* itB;     // [C][224] slot | novf << 8 | ovf0 << 16
+    const float2* tw2;       // [16][16] e^{-2 pi i (i j) / N}
+    const float2* tw448;     // [2N] e^{-2 pi i t / (2N)} (448 entries at N = 224, 512 at N = 256)
+    const uint32_t* itA;     // [C][N] work item of thread tid: k1 | cnt << 8 | start << 16 (cnt == 0: no item)
+    const uint32_t* itB;     // [C][N] slot | novf << 8 | ovf0 << 16
     const uint32_t* ent;     // [nmeas] j | k2 << 16, frame-major, grouped by item
     const uint16_t* rowmask; // [C][16] non-empty rows, by inverse-FFT lane
     int n_ovf;               // overflow partials per frame (sizes the shared-memory slots)
@@ -50,11 +50,12 @@ struct K1Params {
     int mode;
     float inv_1p_rho;
     double rho;              // host side only (general V: selects the precomputed (G_k + rho I)^{-1})
+    int nf;                  // image side N == M: 224 (every kernel) or 256 (streaming kernels only)
 };
 
-int k1_launch(qmri_ctx* ctx, const K1Params& p, int S, int ns_max, int mc);
+int k1_launch(qmri_ctx* ctx, const K1Params& p, int S, int ns_max, int mc);  // cluster kernel: N == M == 224 only
 constexpr int K1_STREAM_MIN_IMAGES_DIV = 8;  // streaming kernels from S * C >= SM count / 8 images on (two 10-channel slices on B200)
-// streaming variant: one CTA per (slice, channel); needs K1Tables::stream_ok
+// streaming variant: G CTAs per (slice, channel); needs K1Tables::stream_ok.  The only x-update kernels for N == 256.
 int k1_stream_groups(int S, int C, int sm_count);
 size_t k1_stream_part_elems(int S, int C, int G, int ns_max);
 size_t k1_stream_cbuf_elems(int S, int C, int ns_max);
@@ -110,6 +111,7 @@ struct GeneralMix {
     const int* meas_u;       // [nmeas]
     const int* meas_frame;   // [nmeas]
     int S, C, L, G, nU, nmeas;
+    float inv_n;             // 1 / N: unitary scaling 1/sqrt(N*M), once per transform direction
 };
 int k1_general_mix_forward(qmri_ctx* ctx, const GeneralMix& m);   // y_i(k) = sum_c V(i,c) Z^_c(k)
 int k1_general_mix_adjoint(qmri_ctx* ctx, const GeneralMix& m);   // cbuf_c(k) = sum_{i: k in Omega_i} V(i,c) y_i(k)

@@ -9,7 +9,8 @@
 // A z is needed only at the <= ~700 sampled k-space locations of the channel and
 // A^H c is the inverse transform of a sparse array, so the m-direction transforms
 // are evaluated as sparse DFT sums, and only the n-direction (contiguous dim) uses
-// full length-224 FFTs (224 = 14 x 16, two register-resident stages).
+// full length-224 FFTs (224 = 14 x 16, two register-resident stages).  The streaming kernels
+// (xupdate_stream.cu) also run N == M == 256 = 16 x 16: see Side below.
 //
 // The functions here are __host__ __device__ so that tests/test_k1_emulation.py can
 // run the exact kernel arithmetic on the CPU (no GPU in the build container).
@@ -28,7 +29,7 @@ static inline float2 make_float2(float a, float b) { return float2{a, b}; }
 
 namespace k1 {
 
-constexpr int NF = 224;   // image side (N == M == 224) and FFT length
+constexpr int NF = 224;   // image side (N == M == 224) and FFT length of the cluster and real-image kernels
 constexpr int CS = 225;   // shared-memory column stride in float2 (odd: conflict-free across columns)
 constexpr int TWP = NF + NF / 16;  // padded twiddle table: entry t sits at t + (t >> 4), so strided lookups spread over banks
 
@@ -151,19 +152,21 @@ QHD void fft_s1_load(const float2* col, int n2, const float2* tw, float2 (&a)[16
 #pragma unroll
     for (int k1 = 1; k1 < 14; ++k1) a[k1] = cmul(a[k1], tw[n2 * k1]);
 }
+// (the stage-1 store and the stage-2 store / loads below are shared with the streaming kernels, which also run N = 256: R = N / 16)
+template <int N = NF>
 QHD void fft_s1_store(float2* col, int n2, const float2 (&a)[16]) {
 #pragma unroll
-    for (int k1 = 0; k1 < 14; ++k1) col[swz(k1, n2)] = a[k1];
+    for (int k1 = 0; k1 < N / 16; ++k1) col[swz(k1, n2)] = a[k1];
 }
 QHD void fft_s2_load(const float2* col, int k1, float2 (&b)[16]) {
 #pragma unroll
     for (int n2 = 0; n2 < 16; ++n2) b[n2] = col[swz(k1, n2)];
     dft16(b);
 }
-template <bool INV>
+template <bool INV, int N = NF>
 QHD void fft_s2_store(float2* col, int k1, const float2 (&b)[16]) {
 #pragma unroll
-    for (int k2 = 0; k2 < 16; ++k2) col[k1 + 14 * k2] = INV ? cswap(b[k2]) : b[k2];
+    for (int k2 = 0; k2 < 16; ++k2) col[k1 + (N / 16) * k2] = INV ? cswap(b[k2]) : b[k2];
 }
 
 // ---- sparse m-direction transforms -------------------------------------------------
@@ -212,18 +215,34 @@ QHD void sparse_idft_flat(float2* col, const float2* c, const float2* twp, const
 
 
 // =====================================================================================
-// Streaming variant (xupdate_stream.cu): one CTA walks the eight 28-column slabs of a
+// Streaming variant (xupdate_stream.cu): one CTA walks the sixteen R-column slabs of a
 // (slice, channel) image one after the other, so no cluster exchange is needed.
-//  * the first forward stage takes its 14 inputs from registers (loaded straight from
-//    global memory), the last inverse stage leaves its 14 outputs in registers (stored
+// Image sides N = 16 R: 224 (R = 14) and 256 (R = 16); the functions below take N as a template
+// argument, and the 224 instance is the arithmetic of the original 224-only kernels.
+//  * the first forward stage takes its R inputs from registers (loaded straight from
+//    global memory), the last inverse stage leaves its R outputs in registers (stored
 //    straight to global memory): two shared-memory passes fewer per transform;
-//  * the inverse transform runs radix 16 first, radix 14 last, so that a half-warp's
+//  * the inverse transform runs radix 16 first, radix R last, so that a half-warp's
 //    outputs n = c + 16 d are 16 consecutive floats in global memory;
 //  * the sparse m-direction sums are evaluated per k-space ROW k1: the thread keeps the
-//    28 slab values of its row in registers and walks the row's samples with a rotating
-//    twiddle (t <- t * e^{-+2 pi i k2 / 224}), so the inner loops touch no shared memory.
-// tw2[i][j] = e^{-2 pi i (i j) / 224}, i, j < 16: stage twiddles, lanes contiguous in j.
+//    R slab values of its row in registers and walks the row's samples with a rotating
+//    twiddle (t <- t * e^{-+2 pi i k2 / N}), so the inner loops touch no shared memory.
+// tw2[i][j] = e^{-2 pi i (i j) / N}, i, j < 16: stage twiddles, lanes contiguous in j.
 // =====================================================================================
+template <int N>
+struct Side {
+    static_assert(N == 224 || N == 256, "streaming kernels: N == M == 224 or 256");
+    static constexpr int R = N / 16;            // radix of the first forward / last inverse stage = columns per slab
+    static constexpr int CS = N + 1;            // shared-memory column stride in float2 (odd: conflict-free across columns)
+    static constexpr int NP = R / 2;            // column pairs per slab in the sparse sums
+    static constexpr int OVF_STRIDE = R + 1;    // float2 per overflow partial (R used; odd stride keeps the lanes on different banks)
+};
+template <int R>
+QHD void dft_r(float2 (&x)[16]) {
+    if constexpr (R == 14) dft14(x);
+    else dft16(x);
+}
+
 constexpr int QMAX_STREAM = 64;      // most samples one work item may carry
 constexpr int OVF_MAX_STREAM = 96;   // most overflow partials (row chunks beyond the first) per frame
 
@@ -239,20 +258,23 @@ QHD float2 ld_ordered(const float2* p) {
 #endif
 }
 
-// forward stage 1 on register inputs: a[n1] = x[16 n1 + n2]
+// forward stage 1 on register inputs: a[n1] = x[16 n1 + n2], n1 < R
+template <int N = NF>
 QHD void fwd_s1_regs(float2 (&a)[16], int n2, const float2* tw2) {
-    dft14(a);
+    constexpr int R = Side<N>::R;
+    dft_r<R>(a);
 #pragma unroll
-    for (int k1 = 1; k1 < 14; ++k1) a[k1] = cmul(a[k1], tw2[16 * k1 + n2]);
+    for (int k1 = 1; k1 < R; ++k1) a[k1] = cmul(a[k1], tw2[16 * k1 + n2]);
 }
 
 // inverse transform of one column via the swap identity  ifft(U) = swap(fft(swap(U))) (unnormalised):
-// input index k = 14 a + b, output index n = c + 16 d
-//   X[c + 16 d] = sum_b w14^{b d} [ w224^{b c} sum_a U[14 a + b] w16^{a c} ]
-// mask: bit a set = row 14 a + b holds samples; the other rows of the sparse k-space array are zero and are not read
+// input index k = R a + b, output index n = c + 16 d
+//   X[c + 16 d] = sum_b wR^{b d} [ wN^{b c} sum_a U[R a + b] w16^{a c} ]
+// mask: bit a set = row R a + b holds samples; the other rows of the sparse k-space array are zero and are not read
+template <int N = NF>
 QHD void inv_s1_load(const float2* col, int b, const float2* tw2, uint32_t mask, float2 (&x)[16]) {
 #pragma unroll
-    for (int a = 0; a < 16; ++a) x[a] = ((mask >> a) & 1u) ? cswap(col[14 * a + b]) : make_float2(0.f, 0.f);
+    for (int a = 0; a < 16; ++a) x[a] = ((mask >> a) & 1u) ? cswap(col[Side<N>::R * a + b]) : make_float2(0.f, 0.f);
     dft16(x);
 #pragma unroll
     for (int c = 1; c < 16; ++c) x[c] = cmul(x[c], ld_ordered(tw2 + 16 * c + b));
@@ -261,44 +283,49 @@ QHD void inv_s1_store(float2* col, int b, const float2 (&x)[16]) {
 #pragma unroll
     for (int c = 0; c < 16; ++c) col[swz(b, c)] = x[c];
 }
-// leaves x[d] = (inverse transform)[c + 16 d], d = 0..13
+// leaves x[d] = (inverse transform)[c + 16 d], d < R
+template <int N = NF>
 QHD void inv_s2_regs(const float2* col, int c, float2 (&x)[16]) {
+    constexpr int R = Side<N>::R;
 #pragma unroll
-    for (int b = 0; b < 14; ++b) x[b] = col[swz(b, c)];
-    dft14(x);
+    for (int b = 0; b < R; ++b) x[b] = col[swz(b, c)];
+    dft_r<R>(x);
 #pragma unroll
-    for (int d = 0; d < 14; ++d) x[d] = cswap(x[d]);
+    for (int d = 0; d < R; ++d) x[d] = cswap(x[d]);
 }
 
 // ---- sparse m-direction sums of the streaming kernel -------------------------------------------------
-// Work item = (k-space row k1, up to Q of the row's samples, one half slab of HC = 14 columns); ent[q] = j | k2 << 16.
-// The 14 columns are taken in pairs mirrored about the centre of the half slab, columns 6 - d' and 7 + d' (d = d' + 1/2):
-//   e^{-i phi (base +- d)} = tc * r_d^{+-1},   tc = e^{-i phi base} (base = m0 + 6.5),   r_d = e^{-i phi d},   phi = 2 pi k2 / 224
-// so with P_d = T[7+d'] + T[6-d'], M_d = T[7+d'] - T[6-d'] (formed once per item) a sample costs 4 FMAs and one twiddle
-// rotation per column PAIR.  tw448[x] = e^{-2 pi i x / 448} supplies the half-integer phases.
-constexpr int HC_STREAM = 14;
-constexpr int NP_STREAM = 7;      // column pairs per half slab
-constexpr int OVF_STRIDE = 15;    // float2 per overflow partial (14 used; odd stride keeps the lanes on different banks)
+// Work item = (k-space row k1, up to Q of the row's samples, one slab of R columns); ent[q] = j | k2 << 16.
+// The R columns are taken in NP = R / 2 pairs mirrored about the centre of the slab, columns NP - 1 - d' and NP + d'
+// (d = d' + 1/2):
+//   e^{-i phi (base +- d)} = tc * r_d^{+-1},   tc = e^{-i phi base} (base = m0 + NP - 1/2),   r_d = e^{-i phi d},   phi = 2 pi k2 / N
+// so with P_d = T[NP+d'] + T[NP-1-d'], M_d = T[NP+d'] - T[NP-1-d'] (formed once per item) a sample costs 4 FMAs and one twiddle
+// rotation per column PAIR.  tw2n[x] = e^{-2 pi i x / (2N)} (448 or 512 entries; K1Params::tw448) supplies the half-integer phases.
+constexpr int HC_STREAM = Side<NF>::R;
+constexpr int NP_STREAM = Side<NF>::NP;          // column pairs per half slab of the real-image kernels
+constexpr int OVF_STRIDE = Side<NF>::OVF_STRIDE;
 
-// forward: pc[j] += sum_mm T[mm][k1] e^{-2 pi i k2 (m0 + mm) / 224} over the 14 columns starting at ws (m0 = first column)
-QHD void p3_item(const float2* ws, int k1, const uint32_t* ent, int cnt, const float2* tw448, int m0, float2* pc) {
+// forward: pc[j] += sum_mm T[mm][k1] e^{-2 pi i k2 (m0 + mm) / N} over the R columns starting at ws (m0 = first column)
+template <int N = NF>
+QHD void p3_item(const float2* ws, int k1, const uint32_t* ent, int cnt, const float2* tw2n, int m0, float2* pc) {
+    constexpr int CS = Side<N>::CS, NP = Side<N>::NP;
     if (cnt == 0) return;
-    float2 Pp[NP_STREAM], Mm[NP_STREAM];
+    float2 Pp[NP], Mm[NP];
 #pragma unroll
-    for (int d = 0; d < NP_STREAM; ++d) {
-        const float2 tp = ws[(7 + d) * CS + k1], tm = ws[(6 - d) * CS + k1];
+    for (int d = 0; d < NP; ++d) {
+        const float2 tp = ws[(NP + d) * CS + k1], tm = ws[(NP - 1 - d) * CS + k1];
         Pp[d] = cadd(tp, tm);
         Mm[d] = csub(tp, tm);
     }
     for (int q = 0; q < cnt; ++q) {
         const uint32_t en = ent[q];
         const int k2 = (int)(en >> 16), j = (int)(en & 0xffffu);
-        float2 r = tw448[k2];          // r_{1/2}
+        float2 r = tw2n[k2];          // r_{1/2}
         const float2 st = cmul(r, r);     // e^{-i phi}
-        const float2 tc = tw448[(k2 * (2 * m0 + 13)) % (2 * NF)];
+        const float2 tc = tw2n[(k2 * (2 * m0 + 2 * NP - 1)) % (2 * N)];
         float ax = 0.f, ay = 0.f;
 #pragma unroll
-        for (int d = 0; d < NP_STREAM; ++d) {
+        for (int d = 0; d < NP; ++d) {
             ax = fmaf(r.x, Pp[d].x, ax);
             ax = fmaf(-r.y, Mm[d].y, ax);
             ay = fmaf(r.x, Pp[d].y, ay);
@@ -311,24 +338,26 @@ QHD void p3_item(const float2* ws, int k1, const uint32_t* ent, int cnt, const f
     }
 }
 
-// inverse, step 1: partial sums of  U[mm] = sum_j c_j e^{+2 pi i k2_j (m0 + mm) / 224}  in the (P, M) basis:
+// inverse, step 1: partial sums of  U[mm] = sum_j c_j e^{+2 pi i k2_j (m0 + mm) / N}  in the (P, M) basis:
 //   SP_d = sum_j u_j Re r_d,  SM_d = sum_j u_j Im r_d,  u_j = c_j conj(tc_j)
-QHD void p4_item_partial(float2 (&SP)[NP_STREAM], float2 (&SM)[NP_STREAM], const uint32_t* ent, int cnt, const float2* tw448, int m0,
+template <int N = NF>
+QHD void p4_item_partial(float2 (&SP)[Side<N>::NP], float2 (&SM)[Side<N>::NP], const uint32_t* ent, int cnt, const float2* tw2n, int m0,
                          const float2* pc) {
+    constexpr int NP = Side<N>::NP;
 #pragma unroll
-    for (int d = 0; d < NP_STREAM; ++d) {
+    for (int d = 0; d < NP; ++d) {
         SP[d] = make_float2(0.f, 0.f);
         SM[d] = make_float2(0.f, 0.f);
     }
     for (int q = 0; q < cnt; ++q) {
         const uint32_t en = ent[q];
         const int k2 = (int)(en >> 16), j = (int)(en & 0xffffu);
-        float2 r = tw448[k2];
+        float2 r = tw2n[k2];
         const float2 st = cmul(r, r);
-        const float2 tc = tw448[(k2 * (2 * m0 + 13)) % (2 * NF)];
+        const float2 tc = tw2n[(k2 * (2 * m0 + 2 * NP - 1)) % (2 * N)];
         const float2 u = cmul(pc[j], make_float2(tc.x, -tc.y));
 #pragma unroll
-        for (int d = 0; d < NP_STREAM; ++d) {
+        for (int d = 0; d < NP; ++d) {
             SP[d].x = fmaf(u.x, r.x, SP[d].x);
             SP[d].y = fmaf(u.y, r.x, SP[d].y);
             SM[d].x = fmaf(u.x, r.y, SM[d].x);
@@ -338,42 +367,47 @@ QHD void p4_item_partial(float2 (&SP)[NP_STREAM], float2 (&SM)[NP_STREAM], const
     }
 }
 // inverse, step 2: a primary item leaves the (P, M) basis and writes its row ...
-QHD void p4_item_store(float2* ws, int k1, const float2 (&SP)[NP_STREAM], const float2 (&SM)[NP_STREAM]) {
+template <int N = NF>
+QHD void p4_item_store(float2* ws, int k1, const float2 (&SP)[Side<N>::NP], const float2 (&SM)[Side<N>::NP]) {
+    constexpr int CS = Side<N>::CS, NP = Side<N>::NP;
 #pragma unroll
-    for (int d = 0; d < NP_STREAM; ++d) {
-        ws[(7 + d) * CS + k1] = make_float2(SP[d].x + SM[d].y, SP[d].y - SM[d].x);   // u conj(r)
-        ws[(6 - d) * CS + k1] = make_float2(SP[d].x - SM[d].y, SP[d].y + SM[d].x);   // u r
+    for (int d = 0; d < NP; ++d) {
+        ws[(NP + d) * CS + k1] = make_float2(SP[d].x + SM[d].y, SP[d].y - SM[d].x);       // u conj(r)
+        ws[(NP - 1 - d) * CS + k1] = make_float2(SP[d].x - SM[d].y, SP[d].y + SM[d].x);   // u r
     }
 }
 // ... and, after a barrier, adds the row's overflow partials in slot order (consecutive slots are OVF_STRIDE apart)
+template <int N = NF>
 QHD void p4_row_add_overflow(float2* ws, int k1, const float2* ovf, int novf) {
-    float2 SP[NP_STREAM], SM[NP_STREAM];
+    constexpr int CS = Side<N>::CS, NP = Side<N>::NP;
+    float2 SP[NP], SM[NP];
 #pragma unroll
-    for (int d = 0; d < NP_STREAM; ++d) {
+    for (int d = 0; d < NP; ++d) {
         SP[d] = ovf[d];
-        SM[d] = ovf[NP_STREAM + d];
+        SM[d] = ovf[NP + d];
     }
     for (int i = 1; i < novf; ++i) {
-        const float2* o = ovf + (size_t)i * OVF_STRIDE;
+        const float2* o = ovf + (size_t)i * Side<N>::OVF_STRIDE;
 #pragma unroll
-        for (int d = 0; d < NP_STREAM; ++d) {
-            const float2 a = o[d], b = o[NP_STREAM + d];
+        for (int d = 0; d < NP; ++d) {
+            const float2 a = o[d], b = o[NP + d];
             SP[d].x += a.x; SP[d].y += a.y;
             SM[d].x += b.x; SM[d].y += b.y;
         }
     }
 #pragma unroll
-    for (int d = 0; d < NP_STREAM; ++d) {
-        float2 up = ws[(7 + d) * CS + k1], um = ws[(6 - d) * CS + k1];
-        ws[(7 + d) * CS + k1] = make_float2(up.x + (SP[d].x + SM[d].y), up.y + (SP[d].y - SM[d].x));
-        ws[(6 - d) * CS + k1] = make_float2(um.x + (SP[d].x - SM[d].y), um.y + (SP[d].y + SM[d].x));
+    for (int d = 0; d < NP; ++d) {
+        float2 up = ws[(NP + d) * CS + k1], um = ws[(NP - 1 - d) * CS + k1];
+        ws[(NP + d) * CS + k1] = make_float2(up.x + (SP[d].x + SM[d].y), up.y + (SP[d].y - SM[d].x));
+        ws[(NP - 1 - d) * CS + k1] = make_float2(um.x + (SP[d].x - SM[d].y), um.y + (SP[d].y + SM[d].x));
     }
 }
-QHD void p4_item_spill(float2* o, const float2 (&SP)[NP_STREAM], const float2 (&SM)[NP_STREAM]) {
+template <int N = NF>
+QHD void p4_item_spill(float2* o, const float2 (&SP)[Side<N>::NP], const float2 (&SM)[Side<N>::NP]) {
 #pragma unroll
-    for (int d = 0; d < NP_STREAM; ++d) {
+    for (int d = 0; d < Side<N>::NP; ++d) {
         o[d] = SP[d];
-        o[NP_STREAM + d] = SM[d];
+        o[Side<N>::NP + d] = SM[d];
     }
 }
 
@@ -535,7 +569,8 @@ QHD void p4r_row_add_overflow(float2* ws, int k1, int h, const float2* ovf, int 
     p4r_store<true>(ws, k1, h, SP, SM);
 }
 
-// item table words (op_tables.h): A = k1 | cnt << 8 | start << 16 (k1 == 255: no item);
+// item table words (op_tables.h): A = k1 | cnt << 8 | start << 16 (cnt == 0: no item - every item carries a sample, and k1 == 255
+//                                     is a real row at N = 256; the no-item word is 255);
 //                                 B = slot | novf << 8 | ovf0 << 16 (slot 0: primary; bits 24-31 unused: rows without samples are
 //                                     skipped by the inverse FFT through the row mask)
 

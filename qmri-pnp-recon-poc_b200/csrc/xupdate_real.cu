@@ -175,7 +175,7 @@ __global__ void __launch_bounds__(THREADS, 4) stream_adjr_kernel(K1RealParams p)
     for (int sl = 0; sl < p.slabs_per_cta; ++sl) {
         const int m0 = (slab0 + sl) * (2 * PC);
         const size_t gi = img + (size_t)(m0 + 2 * col) * NF + l16;
-        if (it_k1 != 255) {
+        if (it_cnt != 0) {
 #pragma unroll 1
             for (int h = 0; h < 2; ++h) {
                 float2 SP[NP_STREAM], SM[NP_STREAM];
@@ -186,7 +186,7 @@ __global__ void __launch_bounds__(THREADS, 4) stream_adjr_kernel(K1RealParams p)
         }
         if (p.n_ovf) {
             __syncthreads();
-            if (it_k1 != 255 && it_slot == 0 && it_novf) {
+            if (it_cnt != 0 && it_slot == 0 && it_novf) {
                 // consecutive overflow slots of a row are 2 * OVF_STRIDE apart (the two half slabs interleave)
 #pragma unroll 1
                 for (int h = 0; h < 2; ++h) p4r_row_add_overflow(ws, it_k1, h, ovf + ((size_t)it_ovf0 * 2 + h) * OVF_STRIDE, it_novf, 2 * OVF_STRIDE);

@@ -10,13 +10,14 @@
 // of eight CTAs; that is the right shape for a handful of slices, but it is bound by shared-memory traffic,
 // cluster barriers and the sparse-DFT table walks.  For batches that fill the machine the update is split
 // at its only global dependency - the <= ~700 sampled k-space values of a channel:
-//   stream_fwd_kernel     grid (G, C, S): 224 / G columns of one image, 14 at a time:  global -> registers ->
+//   stream_fwd_kernel     grid (G, C, S): N / G columns of one image, R = N / 16 at a time:  global -> registers ->
 //                         FFT along n -> sampled DFT along m;  partial sample sums -> `part` (5 KB per CTA)
 //   stream_solve_kernel   grid (C, S): adds the G partials in a fixed order, c = (y - A z) / (1 + rho)
 //   stream_adj_kernel     grid (G, C, S): sparse inverse DFT along m -> inverse FFT along n -> registers ->
 //                         w' = v + corr (+ x on the last iteration) -> global; per-slice min / max
-// No cluster, no DSMEM, CTAs of 224 threads at four per SM, work items small enough that the last wave is
-// short.  The first / last FFT stage works on registers filled from / drained to global memory and the
+// Two instances of each kernel, by image side N == M: 224 (R = 14: CTAs of 224 threads, four per SM) and 256 (R = 16: CTAs of
+// 256 threads, three per SM for the forward kernel and two for the adjoint kernel - see fwd_min_ctas / adj_min_ctas).
+// No cluster, no DSMEM, work items small enough that the last wave is short.  The first / last FFT stage works on registers filled from / drained to global memory and the
 // sparse sums run on per-row work items with rotating twiddles (xupdate_phases.cuh), so the shared-memory
 // traffic is about a third of the cluster kernel's.  HBM traffic per pixel-channel: read w (8 B) + v (4 B)
 // in the forward kernel, read v again (4 B) and write w' (8 B) in the adjoint kernel = 24 B against the
@@ -32,9 +33,15 @@ using namespace k1;
 
 namespace {
 
-constexpr int MC = HC_STREAM;         // 14 columns per slab
-constexpr int THREADS = 16 * MC;      // 224: 14 column FFTs x 16 lanes; in the sparse passes one thread per work item
-constexpr int SLABS = NF / MC;        // 16 slabs per image
+// Per image side N: R = N / 16 columns per slab, N threads = R column FFTs x 16 lanes (in the sparse passes one thread per work
+// item, i.e. per k-space row), 16 slabs per image.
+constexpr int SLABS = 16;
+// CTAs per SM the register allocation is fitted to.  N = 256: the forward kernel fits three (80 registers); the adjoint kernel
+// needs more than 80 (at three it spills the work-item fields it keeps across the slab loop), so it is fitted to two.
+template <int N>
+constexpr int fwd_min_ctas() { return N == 224 ? 4 : 3; }
+template <int N>
+constexpr int adj_min_ctas() { return N == 224 ? 4 : 2; }
 
 __device__ __forceinline__ size_t late_offset(size_t off, float after) {
     size_t r;
@@ -47,8 +54,8 @@ struct Item {
 };
 __device__ __forceinline__ Item decode_item(uint32_t A, uint32_t B) {
     Item it;
-    it.k1 = (int)(A & 0xffu);            // 255: no item
-    it.cnt = (int)((A >> 8) & 0xffu);
+    it.k1 = (int)(A & 0xffu);
+    it.cnt = (int)((A >> 8) & 0xffu);    // 0: no item
     it.start = (int)(A >> 16);
     it.slot = (int)(B & 0xffu);          // 0: primary item of its row
     it.novf = (int)((B >> 8) & 0xffu);
@@ -57,13 +64,14 @@ __device__ __forceinline__ Item decode_item(uint32_t A, uint32_t B) {
 }
 
 // ---------------- forward: partial sums of A z over a group of slabs -------------------------------------
-template <int MODE>
-__global__ void __launch_bounds__(THREADS, 4) stream_fwd_kernel(K1Params p) {
+template <int N, int MODE>
+__global__ void __launch_bounds__(N, fwd_min_ctas<N>()) stream_fwd_kernel(K1Params p) {
+    constexpr int MC = Side<N>::R, CS = Side<N>::CS, THREADS = N;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2* ws = reinterpret_cast<float2*>(smem_raw);                  // [MC][CS] slab workspace
     float2* tw2 = ws + MC * CS;                                        // [16][16]
-    float2* tw448 = tw2 + 256;                                         // [448]
-    float2* pc = tw448 + 2 * NF;                                       // [ns_max] sample accumulators
+    float2* tw448 = tw2 + 256;                                         // [2N]
+    float2* pc = tw448 + 2 * N;                                        // [ns_max] sample accumulators
     uint32_t* s_ent = reinterpret_cast<uint32_t*>(pc + p.ns_max);      // [ns_max]
 
     const int tid = threadIdx.x;
@@ -71,15 +79,15 @@ __global__ void __launch_bounds__(THREADS, 4) stream_fwd_kernel(K1Params p) {
     const int ct = p.shared_mask ? 0 : c;  // table row: the channel's own frame, or the shared union mask (general V)
     const int f0 = p.frame_ptr[ct];
     const int ns = p.frame_ptr[ct + 1] - f0;
-    const size_t img = ((size_t)s * p.C + c) * (size_t)(NF * NF);
+    const size_t img = ((size_t)s * p.C + c) * (size_t)(N * N);
 
     for (int i = tid; i < 256; i += THREADS) tw2[i] = p.tw2[i];
-    for (int i = tid; i < 2 * NF; i += THREADS) tw448[i] = p.tw448[i];
+    for (int i = tid; i < 2 * N; i += THREADS) tw448[i] = p.tw448[i];
     for (int i = tid; i < ns; i += THREADS) {
         s_ent[i] = p.ent[f0 + i];
         pc[i] = make_float2(0.f, 0.f);
     }
-    const uint32_t itA = p.itA[(size_t)ct * NF + tid];
+    const uint32_t itA = p.itA[(size_t)ct * N + tid];
     const int l16 = tid & 15;
     const int col = tid >> 4;
     float2* colp = ws + col * CS;
@@ -90,32 +98,32 @@ __global__ void __launch_bounds__(THREADS, 4) stream_fwd_kernel(K1Params p) {
     for (int sl = 0; sl < p.slabs_per_cta; ++sl) {
         const int m0 = (slab0 + sl) * MC;
         {
-            const size_t gi = img + (size_t)(m0 + col) * NF + l16;
+            const size_t gi = img + (size_t)(m0 + col) * N + l16;
             float2 a[16];
             if (MODE == K1_ADMM) {  // z = 2 v - w
-                float wr[14], wi[14], vv[14];
+                float wr[MC], wi[MC], vv[MC];
 #pragma unroll
-                for (int n1 = 0; n1 < 14; ++n1) {
+                for (int n1 = 0; n1 < MC; ++n1) {
                     wr[n1] = __ldcs(p.in_re + gi + 16 * n1);
                     wi[n1] = __ldcs(p.in_im + gi + 16 * n1);
                     vv[n1] = __ldg(p.v + gi + 16 * n1);
                 }
 #pragma unroll
-                for (int n1 = 0; n1 < 14; ++n1) a[n1] = make_float2(2.f * vv[n1] - wr[n1], -wi[n1]);
+                for (int n1 = 0; n1 < MC; ++n1) a[n1] = make_float2(2.f * vv[n1] - wr[n1], -wi[n1]);
             } else {
 #pragma unroll
-                for (int n1 = 0; n1 < 14; ++n1)
+                for (int n1 = 0; n1 < MC; ++n1)
                     a[n1] = make_float2(__ldcs(p.in_re + gi + 16 * n1), p.in_im ? __ldcs(p.in_im + gi + 16 * n1) : 0.f);
             }
-            fwd_s1_regs(a, l16, tw2);
-            fft_s1_store(colp, l16, a);
+            fwd_s1_regs<N>(a, l16, tw2);
+            fft_s1_store<N>(colp, l16, a);
             __syncwarp();
-            if (l16 < 14) fft_s2_load(colp, l16, a);
+            if (l16 < MC) fft_s2_load(colp, l16, a);
             __syncwarp();
-            if (l16 < 14) fft_s2_store<false>(colp, l16, a);
+            if (l16 < MC) fft_s2_store<false, N>(colp, l16, a);
         }
         __syncthreads();
-        p3_item(ws, (int)(itA & 0xffu), s_ent + (itA >> 16), (int)((itA >> 8) & 0xffu), tw448, m0, pc);
+        p3_item<N>(ws, (int)(itA & 0xffu), s_ent + (itA >> 16), (int)((itA >> 8) & 0xffu), tw448, m0, pc);
         __syncthreads();
     }
     // every sample belongs to exactly one work item, i.e. to one thread: no race on pc above
@@ -124,12 +132,12 @@ __global__ void __launch_bounds__(THREADS, 4) stream_fwd_kernel(K1Params p) {
 }
 
 // ---------------- solve on the samples ----------------------------------------------------------------------
-template <int MODE>
+template <int N, int MODE>
 __global__ void __launch_bounds__(256) stream_solve_kernel(K1Params p) {
     const int c = blockIdx.x, s = blockIdx.y;
     const int f0 = p.frame_ptr[c];
     const int ns = p.frame_ptr[c + 1] - f0;
-    const float inv_n = 1.0f / (float)NF;  // unitary scaling 1/sqrt(N*M), once per transform direction
+    const float inv_n = 1.0f / (float)N;  // unitary scaling 1/sqrt(N*M), once per transform direction
     const float2* part = p.part + ((size_t)s * p.C + c) * p.G * (size_t)p.slot_stride;
     for (int j = threadIdx.x; j < ns; j += blockDim.x) {
         float sx = 0.f, sy = 0.f;
@@ -158,13 +166,14 @@ __global__ void __launch_bounds__(256) stream_solve_kernel(K1Params p) {
 }
 
 // ---------------- adjoint: corr = A^H c, epilogue --------------------------------------------------------------
-template <int MODE>
-__global__ void __launch_bounds__(THREADS, 4) stream_adj_kernel(K1Params p) {
+template <int N, int MODE>
+__global__ void __launch_bounds__(N, adj_min_ctas<N>()) stream_adj_kernel(K1Params p) {
+    constexpr int MC = Side<N>::R, CS = Side<N>::CS, OVF_STRIDE = Side<N>::OVF_STRIDE, THREADS = N;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2* ws = reinterpret_cast<float2*>(smem_raw);                  // [MC][CS]
     float2* tw2 = ws + MC * CS;                                        // [16][16]
-    float2* tw448 = tw2 + 256;                                         // [448]
-    float2* pc = tw448 + 2 * NF;                                       // [ns_max] c
+    float2* tw448 = tw2 + 256;                                         // [2N]
+    float2* pc = tw448 + 2 * N;                                        // [ns_max] c
     float2* ovf = pc + p.ns_max;                                       // [n_ovf][OVF_STRIDE] overflow partials
     uint32_t* s_ent = reinterpret_cast<uint32_t*>(ovf + (size_t)p.n_ovf * OVF_STRIDE);  // [ns_max]
     __shared__ float red_min[THREADS / 32], red_max[THREADS / 32];
@@ -174,20 +183,20 @@ __global__ void __launch_bounds__(THREADS, 4) stream_adj_kernel(K1Params p) {
     const int ct = p.shared_mask ? 0 : c;
     const int f0 = p.frame_ptr[ct];
     const int ns = p.frame_ptr[ct + 1] - f0;
-    const size_t img = ((size_t)s * p.C + c) * (size_t)(NF * NF);
+    const size_t img = ((size_t)s * p.C + c) * (size_t)(N * N);
 
     for (int i = tid; i < 256; i += THREADS) tw2[i] = p.tw2[i];
-    for (int i = tid; i < 2 * NF; i += THREADS) tw448[i] = p.tw448[i];
+    for (int i = tid; i < 2 * N; i += THREADS) tw448[i] = p.tw448[i];
     for (int i = tid; i < ns; i += THREADS) {
         s_ent[i] = p.ent[f0 + i];
         if (MODE == K1_ADJOINT && !p.shared_mask) {
             const float2 y = p.y[(size_t)s * p.nmeas + f0 + i];
-            pc[i] = make_float2(y.x * (1.0f / (float)NF), y.y * (1.0f / (float)NF));
+            pc[i] = make_float2(y.x * (1.0f / (float)N), y.y * (1.0f / (float)N));
         } else {
             pc[i] = p.cbuf[((size_t)s * p.C + c) * p.slot_stride + p.slot_off + i];
         }
     }
-    const uint32_t itA = p.itA[(size_t)ct * NF + tid], itB = p.itB[(size_t)ct * NF + tid];
+    const uint32_t itA = p.itA[(size_t)ct * N + tid], itB = p.itB[(size_t)ct * N + tid];
     const int l16 = tid & 15;
     const uint32_t rmask = p.rowmask[ct * 16 + l16];
     const int col = tid >> 4;
@@ -199,53 +208,53 @@ __global__ void __launch_bounds__(THREADS, 4) stream_adj_kernel(K1Params p) {
 #pragma unroll 1
     for (int sl = 0; sl < p.slabs_per_cta; ++sl) {
         const int m0 = (slab0 + sl) * MC;
-        const size_t gi = img + (size_t)(m0 + col) * NF + l16;
+        const size_t gi = img + (size_t)(m0 + col) * N + l16;
         {
             const Item it = decode_item(itA, itB);
-            if (it.k1 != 255) {
-                float2 SP[NP_STREAM], SM[NP_STREAM];
-                p4_item_partial(SP, SM, s_ent + it.start, it.cnt, tw448, m0, pc);
-                if (it.slot == 0) p4_item_store(ws, it.k1, SP, SM);
-                else p4_item_spill(ovf + (size_t)(it.slot - 1) * OVF_STRIDE, SP, SM);
+            if (it.cnt != 0) {
+                float2 SP[Side<N>::NP], SM[Side<N>::NP];
+                p4_item_partial<N>(SP, SM, s_ent + it.start, it.cnt, tw448, m0, pc);
+                if (it.slot == 0) p4_item_store<N>(ws, it.k1, SP, SM);
+                else p4_item_spill<N>(ovf + (size_t)(it.slot - 1) * OVF_STRIDE, SP, SM);
             }
         }
         if (p.n_ovf) {
             __syncthreads();
             const Item it = decode_item(itA, itB);
-            if (it.k1 != 255 && it.slot == 0 && it.novf) p4_row_add_overflow(ws, it.k1, ovf + (size_t)it.ovf0 * OVF_STRIDE, it.novf);
+            if (it.cnt != 0 && it.slot == 0 && it.novf) p4_row_add_overflow<N>(ws, it.k1, ovf + (size_t)it.ovf0 * OVF_STRIDE, it.novf);
         }
         __syncthreads();
         {
             float2 a[16];
-            if (l16 < 14) inv_s1_load(colp, l16, tw2, rmask, a);
+            if (l16 < MC) inv_s1_load<N>(colp, l16, tw2, rmask, a);
             __syncwarp();
-            if (l16 < 14) inv_s1_store(colp, l16, a);
+            if (l16 < MC) inv_s1_store(colp, l16, a);
             __syncwarp();
-            inv_s2_regs(colp, l16, a);
+            inv_s2_regs<N>(colp, l16, a);
             // What the correction is added to (v in ADMM mode, z in SOLVE mode).  The offset is made to depend on the transform's
-            // last output so that the 14 - 28 loads are not hoisted above it: held across the transform they spill.
-            const size_t gl = late_offset(gi, a[13].y);
-            float br[14], bi[14];
+            // last output so that the R - 2R loads are not hoisted above it: held across the transform they spill.
+            const size_t gl = late_offset(gi, a[MC - 1].y);
+            float br[MC], bi[MC];
             if (MODE == K1_ADMM) {
 #pragma unroll
-                for (int d = 0; d < 14; ++d) br[d] = __ldg(p.v + gl + 16 * d);
+                for (int d = 0; d < MC; ++d) br[d] = __ldg(p.v + gl + 16 * d);
             } else if (MODE == K1_SOLVE) {
 #pragma unroll
-                for (int d = 0; d < 14; ++d) {
+                for (int d = 0; d < MC; ++d) {
                     br[d] = p.in_re[gl + 16 * d];  // plain loads: the general-V accumulation passes run this mode in place (in == out)
                     bi[d] = p.in_im ? p.in_im[gl + 16 * d] : 0.f;
                 }
             }
             if (MODE == K1_ADMM && p.x_re) {  // last iteration: x = z + corr = 2 v - w + corr; w' may overwrite w in place, so x goes first
 #pragma unroll
-                for (int d = 0; d < 14; ++d) {
+                for (int d = 0; d < MC; ++d) {
                     const float wr = __ldcs(p.in_re + gi + 16 * d), wi = __ldcs(p.in_im + gi + 16 * d);
                     p.x_re[gi + 16 * d] = 2.f * br[d] - wr + a[d].x;
                     p.x_im[gi + 16 * d] = a[d].y - wi;
                 }
             }
 #pragma unroll
-            for (int d = 0; d < 14; ++d) {
+            for (int d = 0; d < MC; ++d) {
                 float ore, oim;
                 if (MODE == K1_ADMM) {  // w' = v + corr
                     ore = br[d] + a[d].x;
@@ -287,37 +296,54 @@ __global__ void __launch_bounds__(THREADS, 4) stream_adj_kernel(K1Params p) {
     }
 }
 
-size_t fwd_smem(const K1Params& p) { return (size_t)(MC * CS + 256 + 2 * NF + p.ns_max) * sizeof(float2) + (size_t)p.ns_max * 4 + 16; }
+template <int N>
+size_t fwd_smem(const K1Params& p) {
+    return (size_t)(Side<N>::R * Side<N>::CS + 256 + 2 * N + p.ns_max) * sizeof(float2) + (size_t)p.ns_max * 4 + 16;
+}
+template <int N>
 size_t adj_smem(const K1Params& p) {
-    return (size_t)(MC * CS + 256 + 2 * NF + p.ns_max + (size_t)p.n_ovf * OVF_STRIDE) * sizeof(float2) + (size_t)p.ns_max * 4 + 16;
+    return (size_t)(Side<N>::R * Side<N>::CS + 256 + 2 * N + p.ns_max + (size_t)p.n_ovf * Side<N>::OVF_STRIDE) * sizeof(float2) +
+           (size_t)p.ns_max * 4 + 16;
 }
 
-template <int MODE>
+template <int N, int MODE>
 int launch_mode(qmri_ctx* ctx, const K1Params& p, int S) {
     static size_t conf_f_dev[QMRI_MAX_DEV] = {}, conf_a_dev[QMRI_MAX_DEV] = {};
     size_t &conf_f = conf_f_dev[qmri_dev_slot(ctx)], &conf_a = conf_a_dev[qmri_dev_slot(ctx)];
-    const size_t sf = fwd_smem(p), sa = adj_smem(p);
+    const size_t sf = fwd_smem<N>(p), sa = adj_smem<N>(p);
     if (sf > conf_f) {
-        QCUDA(cudaFuncSetAttribute(stream_fwd_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sf));
+        QCUDA(cudaFuncSetAttribute(stream_fwd_kernel<N, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sf));
         conf_f = sf;
     }
     if (sa > conf_a) {
-        QCUDA(cudaFuncSetAttribute(stream_adj_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sa));
+        QCUDA(cudaFuncSetAttribute(stream_adj_kernel<N, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sa));
         conf_a = sa;
     }
     if (MODE != K1_ADJOINT && !(p.stage & K1_STAGE_ADJ_ONLY)) {
-        stream_fwd_kernel<MODE><<<dim3(p.G, p.C, S), THREADS, sf, ctx->stream>>>(p);
+        stream_fwd_kernel<N, MODE><<<dim3(p.G, p.C, S), N, sf, ctx->stream>>>(p);
         QLAUNCH_CHECK(ctx);
         if (!p.shared_mask && !(p.stage & K1_STAGE_NO_SOLVE)) {  // (the real-state loop runs its own recurrence on the partial sums)
-            stream_solve_kernel<MODE><<<dim3(p.C, S), 256, 0, ctx->stream>>>(p);
+            stream_solve_kernel<N, MODE><<<dim3(p.C, S), 256, 0, ctx->stream>>>(p);
             QLAUNCH_CHECK(ctx);
         }
     }
     if (MODE != K1_FORWARD && !(p.stage & K1_STAGE_FWD_ONLY)) {
-        stream_adj_kernel<MODE><<<dim3(p.G, p.C, S), THREADS, sa, ctx->stream>>>(p);
+        stream_adj_kernel<N, MODE><<<dim3(p.G, p.C, S), N, sa, ctx->stream>>>(p);
         QLAUNCH_CHECK(ctx);
     }
     return QMRI_OK;
+}
+
+template <int N>
+int launch_side(qmri_ctx* ctx, const K1Params& p, int S) {
+    if (adj_smem<N>(p) > 100 * 1024)
+        return qmri_fail(QMRI_EUNSUPPORTED, "x-update (streaming kernel): %zu bytes of shared memory needed", adj_smem<N>(p));
+    switch (p.mode) {
+        case K1_ADMM: return launch_mode<N, K1_ADMM>(ctx, p, S);
+        case K1_SOLVE: return launch_mode<N, K1_SOLVE>(ctx, p, S);
+        case K1_FORWARD: return launch_mode<N, K1_FORWARD>(ctx, p, S);
+        default: return launch_mode<N, K1_ADJOINT>(ctx, p, S);
+    }
 }
 
 }  // namespace
@@ -348,11 +374,7 @@ int k1_stream_launch(qmri_ctx* ctx, const K1Params& p_in, int S, int ns_max) {
         p.slot_off = 0;
         p.slot_stride = ns_max;
     }
-    if (adj_smem(p) > 100 * 1024) return qmri_fail(QMRI_EUNSUPPORTED, "x-update (streaming kernel): %zu bytes of shared memory needed", adj_smem(p));
-    switch (p.mode) {
-        case K1_ADMM: return launch_mode<K1_ADMM>(ctx, p, S);
-        case K1_SOLVE: return launch_mode<K1_SOLVE>(ctx, p, S);
-        case K1_FORWARD: return launch_mode<K1_FORWARD>(ctx, p, S);
-        default: return launch_mode<K1_ADJOINT>(ctx, p, S);
-    }
+    if (p.nf == 224) return launch_side<224>(ctx, p, S);
+    if (p.nf == 256) return launch_side<256>(ctx, p, S);
+    return qmri_fail(QMRI_EUNSUPPORTED, "x-update (streaming kernel): image side %d (224 or 256)", p.nf);
 }
