@@ -184,12 +184,27 @@ int qmri_admm_download(qmri_admm* st, void* x_out, int x_dtype);
 /* Device views of the state after a run: planar fp32 [S][C][M][N]. */
 int qmri_admm_state_dev(qmri_admm* st, const float** x_re, const float** x_im);
 int qmri_admm_destroy(qmri_admm* st);
-/* Kernel-only x-update step on a resident state (w, v) -> w' ; used by bench.py for the K1 roofline. */
+/* Kernel-only x-update step on a resident state (w, v) -> w' ; used by bench.py for the K1 roofline.  With a monitor attached
+ * (qmri_admm_monitor) a complex-state session runs the monitored kernel instances, which write their partial sums but no history
+ * row; a real-state session (QMRI_K1_STATE=real) runs its real-state kernels, which are never monitored. */
 int qmri_admm_xupdate_only(qmri_admm* st, int reps);
 /* Algorithmic HBM bytes per pixel-channel of one x-update in the state formulation this session runs: 8 for the real-state
  * loop (read v, write Re w'; two slices or more, V = eye: csrc/xupdate_real.cu), 20 for the complex-state kernels (read w and v,
  * write w').  bench.py reports the x-update roofline against this figure, never against bytes that do not move. */
 int qmri_admm_xupdate_bytes(qmri_admm* st);
+/* Convergence history, PnP_ADMM.m:106-109: after the x-update of iteration k = 1..iters, per slice s,
+ *   dc_res(k, s) = |y_s - F.forward(x_k,s)| / |y_s|        gt_err(k, s) = |gt_s - x_k,s| / |gt_s|
+ * over all N*M*C entries of the slice (x_k before the denoiser; k = 1 is the solve from X0; a zero denominator gives NaN).
+ * Recorded on the device inside the loop (and its CUDA graph), downloaded once by qmri_admm_history.  Call qmri_admm_monitor
+ * after qmri_admm_create; it holds for every later run until it is called again.  gt: N x M x C x S host array (param.gt_tsmi),
+ * real or complex, any of the four dtypes, or NULL for the residual only; enable = 0 switches monitoring off (the unmonitored
+ * kernels run, unchanged).  A monitored session runs the complex-state streaming x-update at every batch size (general V included):
+ * QMRI_EUNSUPPORTED with QMRI_K1_KERNEL=cluster; QMRI_K1_STATE=real sessions run the complex-state loop while monitored. */
+int qmri_admm_monitor(qmri_admm* st, int enable, const void* gt, int gt_dtype);
+/* History of the last run, MATLAB column-major iters x S doubles.  *iters receives the rows (0 when the last run was not
+ * monitored or ran no iteration); dc_res / gt_err may be NULL (query the size first).  QMRI_EINVAL if gt_err is asked for and the
+ * last run had no ground truth. */
+int qmri_admm_history(qmri_admm* st, double* dc_res, double* gt_err, int* iters);
 
 /* ---- dictionary matching ---------------------------------------------------------
  * Replaces out = mrf_dtm_cpu(dict, data, par)   main_files/dictionary_matching/mrf_dtm_cpu.m:1-166

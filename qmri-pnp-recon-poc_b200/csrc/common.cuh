@@ -106,3 +106,20 @@ __host__ __device__ static inline float ordered_to_float(int k) {
     return f;
 #endif
 }
+
+#ifdef __CUDACC__
+// Sum of v over a block of THREADS threads in a fixed order (a butterfly within each warp, then the warps in order), so that the
+// result does not depend on scheduling: no atomics.  Valid in thread 0.  Every thread of the block must call it.
+template <int THREADS>
+__device__ __forceinline__ double block_sum_fixed(double v) {
+    static_assert(THREADS % 32 == 0, "whole warps");
+    __shared__ double red[THREADS / 32];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    if (threadIdx.x == 0)
+        for (int w = 1; w < THREADS / 32; ++w) v += red[w];
+    return v;
+}
+#endif

@@ -138,6 +138,44 @@ __global__ void minmax_finalize_kernel(int* ord, float* mm, int S) {
 
 inline unsigned nblk(size_t n, int t = 256) { return (unsigned)((n + t - 1) / t); }
 
+// PnP-ADMM progress monitor (PnP_ADMM.m:106-109).  Per-slice sum of squares of a [S][len] (+ b) fp32 array: one block per slice,
+// a fixed summation order (no atomics), so the denominators of the history are the same bits on every run.
+constexpr int MON_THREADS = 256;
+__global__ void __launch_bounds__(MON_THREADS) slice_sumsq_kernel(const float* a, const float* b, size_t len, double* out) {
+    const int s = blockIdx.x;
+    double acc = 0.0;
+    for (size_t i = threadIdx.x; i < len; i += MON_THREADS) {
+        const double u = a[(size_t)s * len + i], w = b ? b[(size_t)s * len + i] : 0.f;
+        acc += u * u + w * w;
+    }
+    acc = block_sum_fixed<MON_THREADS>(acc);
+    if (threadIdx.x == 0) out[s] = acc;
+}
+// Row k of the history from the monitored x-update's partial sums (stream_solve_kernel: [S][C], stream_adj_kernel: [S][C][G]),
+// each slice's summed in a fixed order.  k is a device-side counter, zeroed by qmri_admm_run and advanced here, because a replayed
+// CUDA graph cannot take a new argument per iteration.  One block, so that every slice is written before the counter moves.
+// dc_scale = (rho / (1 + rho))^2 turns |y - A z|^2 into |y - A x|^2.  A zero denominator gives NaN.
+__global__ void __launch_bounds__(MON_THREADS) monitor_finalize_kernel(const double* dc_part, const double* gt_part, const double* y2,
+                                                                       const double* gt2, int* counter, double* h_dc, double* h_gt,
+                                                                       int S, int dc_n, int gt_n, int rows, double dc_scale) {
+    const int k = *counter;
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+    if (k < rows) {
+        for (int s = threadIdx.x; s < S; s += MON_THREADS) {
+            double a = 0.0;
+            for (int i = 0; i < dc_n; ++i) a += dc_part[(size_t)s * dc_n + i];
+            h_dc[(size_t)k * S + s] = y2[s] > 0.0 ? sqrt(a * dc_scale / y2[s]) : nan;
+            if (h_gt) {
+                double b = 0.0;
+                for (int i = 0; i < gt_n; ++i) b += gt_part[(size_t)s * gt_n + i];
+                h_gt[(size_t)k * S + s] = gt2[s] > 0.0 ? sqrt(b / gt2[s]) : nan;
+            }
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) *counter = k + 1;
+}
+
 int unpack_async(qmri_ctx* ctx, const void* dev_raw, int dtype, float* re, float* im, size_t n) {
     if (n == 0) return QMRI_OK;
     int cplx = dtype_is_complex(dtype);
@@ -478,6 +516,11 @@ static int k1_general_dispatch(qmri_op* op, K1Params p, int S, DevBuf* part, Dev
     qmri_ctx* ctx = op->ctx;
     const optab::GeneralTables& g = op->g;
     const int nU = g.nU, P = (int)g.parts.size();
+    // monitored PnP-ADMM session: the residual comes from the per-location solve (mix_residual_kernel), the ground-truth error
+    // from the adjoint launch that completes x
+    double* const mon_dc = p.mon_dc;
+    double* const mon_gt = p.mon_gt;
+    p.mon_dc = p.mon_gt = nullptr;
     p.shared_mask = 1;
     p.G = k1_stream_groups(S, op->C, ctx->sm_count);
     p.slot_stride = nU;
@@ -492,6 +535,7 @@ static int k1_general_dispatch(qmri_op* op, K1Params p, int S, DevBuf* part, Dev
     m.meas_u = op->d_meas_u; m.meas_frame = op->d_meas_frame;
     m.S = S; m.C = op->C; m.L = op->L; m.G = p.G; m.nU = nU; m.nmeas = op->t.nmeas;
     m.inv_n = 1.0f / (float)op->N;
+    m.mon_dc = mon_dc;
     auto use_part = [&](K1Params& q, int pi) {
         const StreamDev& sd = op->gparts[pi];
         q.tw2 = sd.tw2; q.tw448 = sd.tw448; q.itA = sd.itA; q.itB = sd.itB; q.ent = sd.ent; q.rowmask = sd.rowmask;
@@ -521,11 +565,14 @@ static int k1_general_dispatch(qmri_op* op, K1Params p, int S, DevBuf* part, Dev
                 q.x_re = q.x_im = nullptr;
             }
             if (!last) q.minmax = nullptr;  // min / max of the finished image only
+            // x is complete after the last pass: SOLVE mode's output, or ADMM mode's x of a one-part union
+            if (last && (p.mode == K1_SOLVE || (pi == 0 && p.x_re))) q.mon_gt = mon_gt;
             QCHECK(k1_stream_launch(ctx, q, S, ns));
             if (pi > 0 && p.mode == K1_ADMM && p.x_re) {  // last iteration: x receives the same corrections
                 K1Params qx = q;
                 qx.in_re = p.x_re; qx.in_im = p.x_im; qx.out_re = p.x_re; qx.out_im = p.x_im;
                 qx.minmax = nullptr;
+                qx.mon_gt = last ? mon_gt : nullptr;
                 QCHECK(k1_stream_launch(ctx, qx, S, ns));
             }
         }
@@ -549,22 +596,41 @@ static int k1_general_dispatch(qmri_op* op, K1Params p, int S, DevBuf* part, Dev
     }
     QCHECK(forward_all());
     QCHECK(k1_general_mix_solve(ctx, m));
+    if (mon_dc) QCHECK(k1_general_mix_residual(ctx, m));
     return adjoint_all();
+}
+
+// A monitored PnP-ADMM session (qmri_admm_monitor) runs its x-update on the streaming kernels at every batch size: they carry the
+// monitor's reductions, the cluster kernel does not.
+static int k1_monitor_supported(const qmri_op* op) {
+    if (op->general) return QMRI_OK;  // the general-V path always runs the streaming transforms
+    if (op->k1_kernel == 1)
+        return qmri_fail(QMRI_EUNSUPPORTED, "QMRI_K1_KERNEL=cluster: the convergence history (qmri_admm_monitor) is computed by the streaming "
+                         "x-update kernels only");
+    if (!op->t.stream_ok)
+        return qmri_fail(QMRI_EUNSUPPORTED, "qmri_admm_monitor: this mask does not fit the streaming kernel's work-item tables (densest "
+                         "k-space row: %d samples)", op->t.max_row);
+    return QMRI_OK;
 }
 
 static int k1_dispatch(qmri_op* op, const K1Params& p_in, int S, DevBuf* part = nullptr, DevBuf* cbuf = nullptr) {
     K1Params p = p_in;
     if (!part) part = &op->k1_part;
     if (!cbuf) cbuf = &op->k1_cbuf;
+    const bool monitored = p.mon_dc || p.mon_gt;
+    if (monitored) {
+        const int rc = k1_monitor_supported(op);
+        if (rc) return rc;
+    }
     if (op->general) return k1_general_dispatch(op, p, S, part, cbuf);
     qmri_ctx* ctx = op->ctx;
     const bool can_stream = op->t.stream_ok;
     bool stream = can_stream && (long long)S * op->C * K1_STREAM_MIN_IMAGES_DIV >= (long long)ctx->sm_count;
-    if (op->N == 256) {
-        if (op->k1_kernel == 1)
+    if (op->N == 256 || monitored) {
+        if (op->k1_kernel == 1 && op->N == 256)
             return qmri_fail(QMRI_EUNSUPPORTED, "QMRI_K1_KERNEL=cluster: the cluster x-update kernel supports N == M == 224 only (operator is "
                              "%d x %d)", op->N, op->M);
-        stream = true;  // stream_ok: checked when the operator was built
+        stream = true;  // stream_ok: checked when the operator was built (256) or by k1_monitor_supported
     }
     if (op->k1_kernel == 1) stream = false;
     if (op->k1_kernel == 2) {
@@ -834,6 +900,19 @@ struct qmri_admm {
     int graph_chunk = 0, graph_prec = -1;
     int64_t graph_launches = 0;
     bool graph_failed = false;
+    // convergence history (qmri_admm_monitor; PnP_ADMM.m:106-109): partial sums of the monitored x-update kernels, the slices'
+    // |y|^2 and |gt|^2, and the history [rows][S] itself, written in the loop (and in its graph) at the row a device counter names
+    int mon = 0;              // 0 off, 1 residual, 2 residual and ground-truth error
+    bool gt_cplx = false;
+    bool y2_stale = true;     // y was uploaded since |y|^2 was reduced
+    int mon_G = 0;            // slab groups of the adjoint kernel (layout of mon_gt)
+    DevBuf gt_re, gt_im, gt2, y2, mon_dc, mon_gt, hist_dc, hist_gt, hist_ctr;
+    int hist_iters = 0;       // rows the last run recorded
+    bool hist_has_gt = false;
+    // monitor mode, and history buffers (address and capacity: the row limit is a kernel argument), the graph was captured with
+    int graph_mon = -1;
+    const void* graph_hist[2] = {nullptr, nullptr};
+    size_t graph_hist_bytes[2] = {0, 0};
 };
 
 static bool admm_lean_eligible(const qmri_op* op, int S);
@@ -921,6 +1000,8 @@ extern "C" int qmri_admm_destroy(qmri_admm* st) {
     st->v.release(); st->x_re.release(); st->x_im.release(); st->mm_ord.release(); st->mm_f.release();
     st->noise.release(); st->cb_in.release(); st->cb_out.release(); st->k1_part.release(); st->k1_cbuf.release();
     st->v_alt.release(); st->cstate.release(); st->mprev.release();
+    st->gt_re.release(); st->gt_im.release(); st->gt2.release(); st->y2.release(); st->mon_dc.release(); st->mon_gt.release();
+    st->hist_dc.release(); st->hist_gt.release(); st->hist_ctr.release();
     if (st->h_in) cudaFreeHost(st->h_in);
     if (st->h_out) cudaFreeHost(st->h_out);
     if (st->graph) cudaGraphExecDestroy(st->graph);
@@ -953,6 +1034,90 @@ extern "C" int qmri_admm_upload(qmri_admm* st, const void* y, int y_dtype, const
         QCUDA(cudaMemsetAsync(st->mprev.p, 0, st->mprev.bytes, ctx->stream));
     }
     st->uploaded = true;
+    st->y2_stale = true;
+    return QMRI_OK;
+}
+
+extern "C" int qmri_admm_monitor(qmri_admm* st, int enable, const void* gt, int gt_dtype) {
+    if (!st) return qmri_fail(QMRI_EINVAL, "qmri_admm_monitor: null state");
+    if (!enable) {
+        st->mon = 0;
+        return QMRI_OK;
+    }
+    if (gt && !valid_dtype(gt_dtype)) return qmri_fail(QMRI_EINVAL, "qmri_admm_monitor: bad ground-truth dtype %d", gt_dtype);
+    qmri_op* op = st->op;
+    QCHECK(k1_monitor_supported(op));
+    qmri_ctx* ctx = op->ctx;
+    DevSetter ds(ctx->device);
+    const int S = st->S, C = op->C;
+    const size_t n = op->plane() * S;
+    st->mon_G = k1_stream_groups(S, C, ctx->sm_count);
+    const int dc_n = op->general ? k1_general_residual_parts(op->g.nU) : C;
+    QCHECK(st->mon_dc.ensure((size_t)S * dc_n * sizeof(double)));
+    QCHECK(st->y2.ensure((size_t)S * sizeof(double)));
+    QCHECK(st->hist_ctr.ensure(sizeof(int)));
+    if (gt) {
+        st->gt_cplx = dtype_is_complex(gt_dtype);
+        QCHECK(st->gt_re.ensure(n * 4));
+        if (st->gt_cplx) QCHECK(st->gt_im.ensure(n * 4));
+        QCHECK(st->gt2.ensure((size_t)S * sizeof(double)));
+        QCHECK(st->mon_gt.ensure((size_t)S * C * st->mon_G * sizeof(double)));
+        QCHECK(op->stage.ensure(n * dtype_size(gt_dtype)));
+        QCUDA(cudaMemcpyAsync(op->stage.p, gt, n * dtype_size(gt_dtype), cudaMemcpyHostToDevice, ctx->stream));
+        QCHECK(unpack_async(ctx, op->stage.p, gt_dtype, st->gt_re.as<float>(), st->gt_cplx ? st->gt_im.as<float>() : nullptr, n));
+        slice_sumsq_kernel<<<S, MON_THREADS, 0, ctx->stream>>>(st->gt_re.as<float>(), st->gt_cplx ? st->gt_im.as<float>() : nullptr,
+                                                                op->plane(), st->gt2.as<double>());
+        QLAUNCH_CHECK(ctx);
+        QCUDA(cudaStreamSynchronize(ctx->stream));  // the host array may go away after this call
+    }
+    st->mon = gt ? 2 : 1;
+    return QMRI_OK;
+}
+
+extern "C" int qmri_admm_history(qmri_admm* st, double* dc_res, double* gt_err, int* iters) {
+    if (!st || !iters) return qmri_fail(QMRI_EINVAL, "qmri_admm_history: null argument");
+    if (gt_err && !st->hist_has_gt)
+        return qmri_fail(QMRI_EINVAL, "qmri_admm_history: gt_err asked for, but the last run had no ground truth (qmri_admm_monitor)");
+    const int K = st->hist_iters, S = st->S;
+    *iters = K;
+    if (!K || (!dc_res && !gt_err)) return QMRI_OK;
+    DevSetter ds(st->op->ctx->device);
+    std::vector<double> h((size_t)K * S);
+    for (int which = 0; which < 2; ++which) {
+        double* out = which ? gt_err : dc_res;
+        if (!out) continue;
+        const DevBuf& b = which ? st->hist_gt : st->hist_dc;
+        QCUDA(cudaMemcpyAsync(h.data(), b.p, h.size() * sizeof(double), cudaMemcpyDeviceToHost, st->op->ctx->stream));
+        QCUDA(cudaStreamSynchronize(st->op->ctx->stream));
+        for (int k = 0; k < K; ++k)  // device [k][s] -> MATLAB column-major iters x S
+            for (int s = 0; s < S; ++s) out[k + (size_t)K * s] = h[(size_t)k * S + s];
+    }
+    return QMRI_OK;
+}
+
+// the monitor's arguments of one x-update (null when the session is not monitored)
+static void admm_mon_params(const qmri_admm* st, K1Params& p) {
+    if (!st->mon) return;
+    p.mon_dc = st->mon_dc.as<double>();
+    if (st->mon == 2) {
+        p.mon_gt = st->mon_gt.as<double>();
+        p.gt_re = st->gt_re.as<float>();
+        p.gt_im = st->gt_cplx ? st->gt_im.as<float>() : nullptr;
+    }
+}
+
+static int admm_mon_finalize(qmri_admm* st) {
+    if (!st->mon) return QMRI_OK;
+    qmri_op* op = st->op;
+    // identity V: the solve kernel's partials are |y - A z|^2 and |y - A x| = rho / (1 + rho) |y - A z|; general V: |y - A x|^2
+    const double f = op->general ? 1.0 : st->prm.gamma / (1.0 + st->prm.gamma);
+    const int rows = (int)(st->hist_dc.bytes / (sizeof(double) * st->S));
+    const int dc_n = op->general ? k1_general_residual_parts(op->g.nU) : op->C;
+    monitor_finalize_kernel<<<1, MON_THREADS, 0, op->ctx->stream>>>(
+        st->mon_dc.as<double>(), st->mon == 2 ? st->mon_gt.as<double>() : nullptr, st->y2.as<double>(), st->gt2.as<double>(),
+        st->hist_ctr.as<int>(), st->hist_dc.as<double>(), st->mon == 2 ? st->hist_gt.as<double>() : nullptr, st->S, dc_n,
+        op->C * st->mon_G, rows, f * f);
+    QLAUNCH_CHECK(op->ctx);
     return QMRI_OK;
 }
 
@@ -966,12 +1131,15 @@ static int admm_k1(qmri_admm* st, bool write_x) {
     p.v = st->v.as<float>();
     p.out_re = st->w_re.as<float>();  // in place: every cluster reads its whole tile before it writes it
     p.out_im = st->w_im.as<float>();
+    // general V with a ground truth: x is written on every iteration, and the launch that completes it sums |gt - x|^2
+    write_x = write_x || (op->general && st->mon == 2);
     p.x_re = write_x ? st->x_re.as<float>() : nullptr;
     p.x_im = write_x ? st->x_im.as<float>() : nullptr;
     p.y = st->y.as<float2>();
     p.minmax = st->mm_ord.as<int>();
     p.inv_1p_rho = (float)(1.0 / (1.0 + st->prm.gamma));
     p.rho = st->prm.gamma;
+    admm_mon_params(st, p);
     return k1_dispatch(op, p, st->S, &st->k1_part, &st->k1_cbuf);
 }
 
@@ -1145,7 +1313,21 @@ extern "C" int qmri_admm_run(qmri_admm* st, int iters) {
     QCUDA(cudaMemcpyAsync(st->x_re.p, st->x0_re.p, n * 4, cudaMemcpyDeviceToDevice, ctx->stream));
     QCUDA(cudaMemcpyAsync(st->x_im.p, st->x0_im.p, n * 4, cudaMemcpyDeviceToDevice, ctx->stream));
     QCHECK(k1_minmax_init(ctx, st->mm_ord.as<int>(), S));
-    const bool lean = st->lean;
+    st->hist_iters = st->mon ? iters : 0;
+    st->hist_has_gt = st->mon == 2;
+    if (st->mon) {  // history rows for this run, sized before any graph capture; row counter back to 0
+        QCHECK(st->hist_dc.ensure((size_t)std::max(iters, 1) * S * sizeof(double)));
+        if (st->mon == 2) QCHECK(st->hist_gt.ensure(st->hist_dc.bytes));
+        if (st->y2_stale) {
+            slice_sumsq_kernel<<<S, MON_THREADS, 0, ctx->stream>>>(reinterpret_cast<const float*>(st->y.p), nullptr,
+                                                                    2 * (size_t)op->t.nmeas, st->y2.as<double>());
+            QLAUNCH_CHECK(ctx);
+            st->y2_stale = false;
+        }
+        QCUDA(cudaMemsetAsync(st->hist_ctr.p, 0, sizeof(int), ctx->stream));
+    }
+    // the real-state loop never forms x: a monitored session runs the complex-state loop
+    const bool lean = st->lean && !st->mon;
     auto iteration = [&](int k) -> int {
         // real-state loop: the denoiser output of the second-to-last iteration goes to a second buffer, because the last
         // x-update needs v_{K-2} next to v_{K-1}
@@ -1175,6 +1357,7 @@ extern "C" int qmri_admm_run(qmri_admm* st, int iters) {
             p.minmax = st->mm_ord.as<int>();
             p.inv_1p_rho = (float)(1.0 / (1.0 + st->prm.gamma));
             p.rho = st->prm.gamma;
+            admm_mon_params(st, p);
             QCHECK(k1_dispatch(op, p, S, &st->k1_part, &st->k1_cbuf));
             if (iters == 1) {  // x_1 is the result
                 QCUDA(cudaMemcpyAsync(st->x_re.p, st->w_re.p, n * 4, cudaMemcpyDeviceToDevice, ctx->stream));
@@ -1183,6 +1366,7 @@ extern "C" int qmri_admm_run(qmri_admm* st, int iters) {
         } else {
             QCHECK(admm_k1(st, k == iters - 1));
         }
+        QCHECK(admm_mon_finalize(st));  // PnP_ADMM.m:106-109: row k of the history
         // PnP_ADMM.m:121-144 also denoise after the last x-update, but only x is returned (:148): v and u of the last iteration
         // are dead, so the final 64-layer forward is skipped
         if (k == iters - 1) return QMRI_OK;
@@ -1199,8 +1383,13 @@ extern "C" int qmri_admm_run(qmri_admm* st, int iters) {
             QCHECK(iteration(k));
             continue;
         }
-        if (st->graph && (st->graph_ws != net->ws || st->graph_chunk != net->chunk || st->graph_prec != net->precision)) {
-            cudaGraphExecDestroy(st->graph);  // the denoiser workspace moved or its mode changed since the capture
+        const int mon_key = st->mon | (st->mon == 2 && st->gt_cplx ? 4 : 0);
+        if (st->graph && (st->graph_ws != net->ws || st->graph_chunk != net->chunk || st->graph_prec != net->precision ||
+                          st->graph_mon != mon_key ||
+                          (st->mon && (st->graph_hist[0] != st->hist_dc.p || st->graph_hist[1] != st->hist_gt.p ||
+                                       st->graph_hist_bytes[0] != st->hist_dc.bytes || st->graph_hist_bytes[1] != st->hist_gt.bytes)))) {
+            // the denoiser workspace moved or its mode changed since the capture, monitoring was switched, or the history moved
+            cudaGraphExecDestroy(st->graph);
             st->graph = nullptr;
         }
         if (!st->graph) {
@@ -1231,6 +1420,11 @@ extern "C" int qmri_admm_run(qmri_admm* st, int iters) {
             st->graph_ws = net->ws;
             st->graph_chunk = net->chunk;
             st->graph_prec = net->precision;
+            st->graph_mon = mon_key;
+            st->graph_hist[0] = st->hist_dc.p;
+            st->graph_hist[1] = st->hist_gt.p;
+            st->graph_hist_bytes[0] = st->hist_dc.bytes;
+            st->graph_hist_bytes[1] = st->hist_gt.bytes;
         }
         QCUDA(cudaGraphLaunch(st->graph, ctx->stream));
         ctx->launches += st->graph_launches;  // kernels inside the replayed graph

@@ -110,7 +110,54 @@ __global__ void __launch_bounds__(128) mix_solve_kernel(GeneralMix m) {
         }
 }
 
+// PnP_ADMM.m:106-107 for general V (monitored sessions): the data-consistency residual of the solved x, per union location
+// r_i(k) = y_i(k) - V(i,:) (Z^(k) + delta(k)) for every frame i sampling k, with delta = cbuf / inv_n (mix_solve_kernel pre-scales it
+// for the inverse transform).  One double partial per block, reduced in a fixed order: no atomics.  A kernel of its own, so that
+// mix_solve_kernel stays as it was for unmonitored sessions.
+constexpr int RES_THREADS = 128;
+__global__ void __launch_bounds__(RES_THREADS) mix_residual_kernel(GeneralMix m) {
+    const int u = blockIdx.x * blockDim.x + threadIdx.x, s = blockIdx.y;
+    double acc = 0.0;
+    if (u < m.nU) {
+        float xx[CMAX], xy[CMAX];
+        const float rs = 1.0f / m.inv_n;
+#pragma unroll
+        for (int c = 0; c < CMAX; ++c) {
+            xx[c] = xy[c] = 0.f;
+            if (c < m.C) {
+                const float2 z = zhat(m, s, c, u);
+                const float2 d = m.cbuf[((size_t)s * m.C + c) * m.nU + u];
+                xx[c] = z.x + d.x * rs;
+                xy[c] = z.y + d.y * rs;
+            }
+        }
+        for (int e = m.memb_ptr[u]; e < m.memb_ptr[u + 1]; ++e) {
+            const float2 y = m.y[(size_t)s * m.nmeas + m.memb_meas[e]];
+            const float* v = m.V + (size_t)m.memb_frame[e] * m.C;
+            double rx = y.x, ry = y.y;
+#pragma unroll
+            for (int c = 0; c < CMAX; ++c)
+                if (c < m.C) {
+                    rx -= (double)v[c] * xx[c];
+                    ry -= (double)v[c] * xy[c];
+                }
+            acc += rx * rx + ry * ry;
+        }
+    }
+    acc = block_sum_fixed<RES_THREADS>(acc);
+    if (threadIdx.x == 0) m.mon_dc[(size_t)s * gridDim.x + blockIdx.x] = acc;
+}
+
 }  // namespace
+
+int k1_general_residual_parts(int nU) { return (nU + RES_THREADS - 1) / RES_THREADS; }
+int k1_general_mix_residual(qmri_ctx* ctx, const GeneralMix& m) {
+    if (m.S == 0) return QMRI_OK;
+    if (m.nU == 0) return qmri_fail(QMRI_EINVAL, "general V: empty union mask");
+    mix_residual_kernel<<<dim3(k1_general_residual_parts(m.nU), m.S), RES_THREADS, 0, ctx->stream>>>(m);
+    QLAUNCH_CHECK(ctx);
+    return QMRI_OK;
+}
 
 int k1_general_mix_forward(qmri_ctx* ctx, const GeneralMix& m) {
     if (m.nmeas == 0 || m.S == 0) return QMRI_OK;

@@ -51,6 +51,12 @@ struct K1Params {
     float inv_1p_rho;
     double rho;              // host side only (general V: selects the precomputed (G_k + rho I)^{-1})
     int nf;                  // image side N == M: 224 (every kernel) or 256 (streaming kernels only)
+    // PnP-ADMM progress monitor (qmri_admm_monitor; streaming kernels, modes ADMM and SOLVE): the monitored kernel instances write
+    // double partial sums, each reduced in a fixed order.  Null: the unmonitored instances run.
+    double* mon_dc;          // [S][C] sum over the channel's samples of |y - A z|^2 (stream_solve_kernel; general V: GeneralMix)
+    double* mon_gt;          // [S][C][G] sum over the CTA's pixels of |gt - x|^2 (stream_adj_kernel; needs gt_re)
+    const float* gt_re;      // [S][C][M][N] ground truth
+    const float* gt_im;      // optional imaginary plane (null: real ground truth)
 };
 
 int k1_launch(qmri_ctx* ctx, const K1Params& p, int S, int ns_max, int mc);  // cluster kernel: N == M == 224 only
@@ -112,7 +118,11 @@ struct GeneralMix {
     const int* meas_frame;   // [nmeas]
     int S, C, L, G, nU, nmeas;
     float inv_n;             // 1 / N: unitary scaling 1/sqrt(N*M), once per transform direction
+    double* mon_dc;          // monitored PnP-ADMM sessions: [S][k1_general_residual_parts(nU)] partial sums of |y - A x|^2
 };
 int k1_general_mix_forward(qmri_ctx* ctx, const GeneralMix& m);   // y_i(k) = sum_c V(i,c) Z^_c(k)
 int k1_general_mix_adjoint(qmri_ctx* ctx, const GeneralMix& m);   // cbuf_c(k) = sum_{i: k in Omega_i} V(i,c) y_i(k)
 int k1_general_mix_solve(qmri_ctx* ctx, const GeneralMix& m);     // cbuf(k) = (G_k + rho I)^{-1} sum_i V(i,:)^T (y_i(k) - V(i,:) Z^(k))
+// after mix_solve: sum over the union locations of a block of sum_i |y_i(k) - V(i,:) X^(k)|^2, X^ = Z^ + delta -> m.mon_dc
+int k1_general_mix_residual(qmri_ctx* ctx, const GeneralMix& m);
+int k1_general_residual_parts(int nU);

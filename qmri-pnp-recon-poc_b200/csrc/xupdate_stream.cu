@@ -42,11 +42,21 @@ template <int N>
 constexpr int fwd_min_ctas() { return N == 224 ? 4 : 3; }
 template <int N>
 constexpr int adj_min_ctas() { return N == 224 ? 4 : 2; }
+// The monitored SOLVE instance (the first x-update of a monitored PnP-ADMM run, once per run) is fitted to one CTA less at 224:
+// at four its ground-truth loads add spills.
+template <int N, int MODE, bool MON>
+constexpr int adj_min_ctas_mon() { return MON && MODE == K1_SOLVE && N == 224 ? 3 : adj_min_ctas<N>(); }
 
 __device__ __forceinline__ size_t late_offset(size_t off, float after) {
     size_t r;
     asm volatile("mov.u64 %0, %1;" : "=l"(r) : "l"(off), "f"(after));
     return r;
+}
+
+template <int THREADS>
+__device__ __forceinline__ double* mon_slot() {
+    __shared__ double slot[THREADS];
+    return slot + threadIdx.x;
 }
 
 struct Item {
@@ -132,13 +142,18 @@ __global__ void __launch_bounds__(N, fwd_min_ctas<N>()) stream_fwd_kernel(K1Para
 }
 
 // ---------------- solve on the samples ----------------------------------------------------------------------
-template <int N, int MODE>
-__global__ void __launch_bounds__(256) stream_solve_kernel(K1Params p) {
+// MON (monitored PnP-ADMM sessions, modes ADMM and SOLVE): also sum |y - A z|^2 over the channel's samples into mon_dc[s][c].  With
+// x = z + A^H c, c = (y - A z) / (1 + rho) and A A^H = I, y - A x = (y - A z) - c = rho c, so |y - A x| = rho / (1 + rho) |y - A z|
+// (the finalize kernel applies the factor): the data-consistency residual of PnP_ADMM.m:106-107 costs no transform.
+constexpr int SOLVE_THREADS = 256;
+template <int N, int MODE, bool MON>
+__global__ void __launch_bounds__(SOLVE_THREADS) stream_solve_kernel(K1Params p) {
     const int c = blockIdx.x, s = blockIdx.y;
     const int f0 = p.frame_ptr[c];
     const int ns = p.frame_ptr[c + 1] - f0;
     const float inv_n = 1.0f / (float)N;  // unitary scaling 1/sqrt(N*M), once per transform direction
     const float2* part = p.part + ((size_t)s * p.C + c) * p.G * (size_t)p.slot_stride;
+    double dc = 0.0;
     for (int j = threadIdx.x; j < ns; j += blockDim.x) {
         float sx = 0.f, sy = 0.f;
 #pragma unroll 1
@@ -152,6 +167,8 @@ __global__ void __launch_bounds__(256) stream_solve_kernel(K1Params p) {
                 sy += t[i].y;
             }
         }
+        const float rx = sx, ry = sy;  // MON: the unscaled sums, so that the monitor adds no use of the scaled ones below (which
+                                       // would stop the compiler from fusing their scaling into the subtraction: different bits)
         sx *= inv_n;
         sy *= inv_n;
         const size_t yi = (size_t)s * p.nmeas + f0 + j;
@@ -161,13 +178,24 @@ __global__ void __launch_bounds__(256) stream_solve_kernel(K1Params p) {
             const float2 y = p.y[yi];
             const float gsc = p.inv_1p_rho * inv_n;  // (y - A z)/(1 + rho), pre-scaled for the inverse transform
             p.cbuf[((size_t)s * p.C + c) * p.slot_stride + j] = make_float2((y.x - sx) * gsc, (y.y - sy) * gsc);
+            if (MON) {
+                const double dr = (double)y.x - (double)rx * inv_n, di = (double)y.y - (double)ry * inv_n;
+                dc += dr * dr + di * di;
+            }
         }
+    }
+    if (MON) {
+        dc = block_sum_fixed<SOLVE_THREADS>(dc);
+        if (threadIdx.x == 0) p.mon_dc[(size_t)s * p.C + c] = dc;
     }
 }
 
 // ---------------- adjoint: corr = A^H c, epilogue --------------------------------------------------------------
-template <int N, int MODE>
-__global__ void __launch_bounds__(N, adj_min_ctas<N>()) stream_adj_kernel(K1Params p) {
+// MON (monitored PnP-ADMM sessions with a ground truth, modes ADMM and SOLVE): also sum |gt - x|^2 over the CTA's pixels into
+// mon_gt[s][c][g] (PnP_ADMM.m:108-109).  ADMM mode forms x = 2 v - w + corr on every iteration, with the expression the
+// last-iteration store uses, so the history of iteration k is the norm of what a k-iteration run returns.
+template <int N, int MODE, bool MON>
+__global__ void __launch_bounds__(N, adj_min_ctas_mon<N, MODE, MON>()) stream_adj_kernel(K1Params p) {
     constexpr int MC = Side<N>::R, CS = Side<N>::CS, OVF_STRIDE = Side<N>::OVF_STRIDE, THREADS = N;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2* ws = reinterpret_cast<float2*>(smem_raw);                  // [MC][CS]
@@ -204,6 +232,9 @@ __global__ void __launch_bounds__(N, adj_min_ctas<N>()) stream_adj_kernel(K1Para
     __syncthreads();
 
     float lmin = INFINITY, lmax = -INFINITY;
+    // MON: this thread's sum of |gt - x|^2, kept in shared memory rather than in the two registers a double takes (the kernel
+    // is at its register limit)
+    if (MON) *mon_slot<THREADS>() = 0.0;
     const int slab0 = g * p.slabs_per_cta;
 #pragma unroll 1
     for (int sl = 0; sl < p.slabs_per_cta; ++sl) {
@@ -245,7 +276,7 @@ __global__ void __launch_bounds__(N, adj_min_ctas<N>()) stream_adj_kernel(K1Para
                     bi[d] = p.in_im ? p.in_im[gl + 16 * d] : 0.f;
                 }
             }
-            if (MODE == K1_ADMM && p.x_re) {  // last iteration: x = z + corr = 2 v - w + corr; w' may overwrite w in place, so x goes first
+            if (MODE == K1_ADMM && !MON && p.x_re) {  // last iteration: x = z + corr = 2 v - w + corr; w' may overwrite w in place, so x goes first
 #pragma unroll
                 for (int d = 0; d < MC; ++d) {
                     const float wr = __ldcs(p.in_re + gi + 16 * d), wi = __ldcs(p.in_im + gi + 16 * d);
@@ -253,6 +284,7 @@ __global__ void __launch_bounds__(N, adj_min_ctas<N>()) stream_adj_kernel(K1Para
                     p.x_im[gi + 16 * d] = a[d].y - wi;
                 }
             }
+            float ge = 0.f;
 #pragma unroll
             for (int d = 0; d < MC; ++d) {
                 float ore, oim;
@@ -266,13 +298,32 @@ __global__ void __launch_bounds__(N, adj_min_ctas<N>()) stream_adj_kernel(K1Para
                     ore = a[d].x;
                     oim = a[d].y;
                 }
+                if (MON) {
+                    float xr = ore, xi = oim;  // SOLVE: x is the output
+                    if (MODE == K1_ADMM) {     // x = 2 v - w + corr, element by element ahead of the in-place store of w'
+                        const float wr = __ldcs(p.in_re + gi + 16 * d), wi = __ldcs(p.in_im + gi + 16 * d);
+                        xr = 2.f * br[d] - wr + a[d].x;
+                        xi = a[d].y - wi;
+                        if (p.x_re) {
+                            p.x_re[gi + 16 * d] = xr;
+                            p.x_im[gi + 16 * d] = xi;
+                        }
+                    }
+                    const float er = __ldcs(p.gt_re + gi + 16 * d) - xr, ei = (p.gt_im ? __ldcs(p.gt_im + gi + 16 * d) : 0.f) - xi;
+                    ge += er * er + ei * ei;
+                }
                 p.out_re[gi + 16 * d] = ore;
                 p.out_im[gi + 16 * d] = oim;
                 lmin = fminf(lmin, ore);
                 lmax = fmaxf(lmax, ore);
             }
+            if (MON) *mon_slot<THREADS>() += ge;
         }
         __syncthreads();
+    }
+    if (MON) {  // one partial per CTA, no atomics: graph replays and direct launches give the same bits
+        const double t = block_sum_fixed<THREADS>(*mon_slot<THREADS>());
+        if (tid == 0) p.mon_gt[((size_t)s * p.C + c) * p.G + g] = t;
     }
     if (p.minmax) {
 #pragma unroll
@@ -306,30 +357,42 @@ size_t adj_smem(const K1Params& p) {
            (size_t)p.ns_max * 4 + 16;
 }
 
+template <int N, int MODE, bool MON>
+int launch_adj(qmri_ctx* ctx, const K1Params& p, int S) {
+    static size_t conf_dev[QMRI_MAX_DEV] = {};
+    size_t& conf = conf_dev[qmri_dev_slot(ctx)];
+    const size_t sa = adj_smem<N>(p);
+    if (sa > conf) {
+        QCUDA(cudaFuncSetAttribute(stream_adj_kernel<N, MODE, MON>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sa));
+        conf = sa;
+    }
+    stream_adj_kernel<N, MODE, MON><<<dim3(p.G, p.C, S), N, sa, ctx->stream>>>(p);
+    QLAUNCH_CHECK(ctx);
+    return QMRI_OK;
+}
+
 template <int N, int MODE>
 int launch_mode(qmri_ctx* ctx, const K1Params& p, int S) {
-    static size_t conf_f_dev[QMRI_MAX_DEV] = {}, conf_a_dev[QMRI_MAX_DEV] = {};
-    size_t &conf_f = conf_f_dev[qmri_dev_slot(ctx)], &conf_a = conf_a_dev[qmri_dev_slot(ctx)];
-    const size_t sf = fwd_smem<N>(p), sa = adj_smem<N>(p);
+    constexpr bool CAN_MON = MODE == K1_ADMM || MODE == K1_SOLVE;
+    static size_t conf_f_dev[QMRI_MAX_DEV] = {};
+    size_t& conf_f = conf_f_dev[qmri_dev_slot(ctx)];
+    const size_t sf = fwd_smem<N>(p);
     if (sf > conf_f) {
         QCUDA(cudaFuncSetAttribute(stream_fwd_kernel<N, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sf));
         conf_f = sf;
-    }
-    if (sa > conf_a) {
-        QCUDA(cudaFuncSetAttribute(stream_adj_kernel<N, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sa));
-        conf_a = sa;
     }
     if (MODE != K1_ADJOINT && !(p.stage & K1_STAGE_ADJ_ONLY)) {
         stream_fwd_kernel<N, MODE><<<dim3(p.G, p.C, S), N, sf, ctx->stream>>>(p);
         QLAUNCH_CHECK(ctx);
         if (!p.shared_mask && !(p.stage & K1_STAGE_NO_SOLVE)) {  // (the real-state loop runs its own recurrence on the partial sums)
-            stream_solve_kernel<N, MODE><<<dim3(p.C, S), 256, 0, ctx->stream>>>(p);
+            if (CAN_MON && p.mon_dc) stream_solve_kernel<N, MODE, CAN_MON><<<dim3(p.C, S), SOLVE_THREADS, 0, ctx->stream>>>(p);
+            else stream_solve_kernel<N, MODE, false><<<dim3(p.C, S), SOLVE_THREADS, 0, ctx->stream>>>(p);
             QLAUNCH_CHECK(ctx);
         }
     }
     if (MODE != K1_FORWARD && !(p.stage & K1_STAGE_FWD_ONLY)) {
-        stream_adj_kernel<N, MODE><<<dim3(p.G, p.C, S), N, sa, ctx->stream>>>(p);
-        QLAUNCH_CHECK(ctx);
+        if (CAN_MON && p.mon_gt) return launch_adj<N, MODE, CAN_MON>(ctx, p, S);
+        return launch_adj<N, MODE, false>(ctx, p, S);
     }
     return QMRI_OK;
 }
@@ -370,6 +433,11 @@ int k1_stream_launch(qmri_ctx* ctx, const K1Params& p_in, int S, int ns_max) {
     p.ns_max = ns_max;
     if (p.G < 1 || SLABS % p.G || !p.part || !p.cbuf) return qmri_fail(QMRI_EINVAL, "x-update (streaming kernel): bad slab grouping / scratch");
     p.slabs_per_cta = SLABS / p.G;
+    // monitoring: the residual partials need the solve kernel (identity V, whole x-update); the ground-truth partials an adjoint
+    // launch that completes x (general V: the last adjoint-only pass)
+    if ((p.mon_dc && (p.shared_mask || p.stage)) || ((p.mon_dc || p.mon_gt) && p.mode != K1_ADMM && p.mode != K1_SOLVE) ||
+        (p.mon_gt && (!p.gt_re || (p.stage & K1_STAGE_FWD_ONLY))))
+        return qmri_fail(QMRI_EINVAL, "x-update (streaming kernel): bad monitor arguments");
     if (!p.shared_mask) {
         p.slot_off = 0;
         p.slot_stride = ns_max;

@@ -161,7 +161,6 @@ int feval_denoiser(void* user, const float* v_in, float* v_out, int H, int W, in
 }  // namespace
 
 extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
-    (void)nlhs;
     if (nrhs < 1) mexErrMsgIdAndTxt("qmri:usage", "qmri_b200_mex(command, ...)");
     char* c = mxArrayToString(prhs[0]);
     std::string cmd = c ? c : "";
@@ -276,7 +275,7 @@ extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* 
         mwSize od[4] = {d[0], d[1], 10, (mwSize)S};
         plhs[0] = mxCreateNumericArray(4, od, mxIsDouble(prhs[2]) ? mxDOUBLE_CLASS : mxSINGLE_CLASS, mxREAL);
         check(qmri_unetres_denoise(net, mxGetData(prhs[2]), dtype_of(prhs[2]), mxGetData(plhs[0]), dtype_of(plhs[0]), S, (int)d[0], (int)d[1]));
-    } else if (cmd == "pnp_admm") {                          // (op, y, param struct) -> x ; param.net = net handle or function handle
+    } else if (cmd == "pnp_admm") {                          // (op, y, param struct) -> x [, info] ; param.net = net handle or function handle
         need(4);
         qmri_op* op = handle_in<qmri_op>(prhs[1]);
         const mxArray* prm = prhs[3];
@@ -312,8 +311,39 @@ extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* 
         mwSize od[4] = {d[0], d[1], (mwSize)dim_of(X0, 2), (mwSize)S};
         CplxIn y(prhs[2]), x0(X0);
         CplxOut x(4, od, mxDOUBLE_CLASS);
-        check(qmri_pnp_admm(op, y.p, y.dtype, x0.p, x0.dtype, S, &p, x.p, QMRI_C128));
-        plhs[0] = x.finish();
+        if (nlhs < 2) {
+            check(qmri_pnp_admm(op, y.p, y.dtype, x0.p, x0.dtype, S, &p, x.p, QMRI_C128));
+            plhs[0] = x.finish();
+        } else {  // [x, info]: the session API with the convergence history of PnP_ADMM.m:106-109 (info.dc_res, info.gt_err: iter x S)
+            const mxArray* gt = mxGetField(prm, 0, "gt_tsmi");
+            if (gt && mxGetNumberOfElements(gt) == 0) gt = nullptr;
+            if (gt && mxGetNumberOfElements(gt) != mxGetNumberOfElements(X0))
+                mexErrMsgIdAndTxt("qmri:param", "param.gt_tsmi must have the size of param.X0");
+            std::vector<CplxIn> g;
+            if (gt) g.emplace_back(gt);
+            qmri_admm* st = nullptr;
+            check(qmri_admm_create(op, S, &p, &st));
+            int K = 0;
+            int r = qmri_admm_monitor(st, 1, gt ? g[0].p : nullptr, gt ? g[0].dtype : QMRI_F64);
+            if (!r) r = qmri_admm_upload(st, y.p, y.dtype, x0.p, x0.dtype);
+            if (!r) r = qmri_admm_run(st, p.iters);
+            if (!r) r = qmri_admm_download(st, x.p, QMRI_C128);
+            if (!r) r = qmri_admm_history(st, nullptr, nullptr, &K);
+            mxArray* dc = mxCreateNumericMatrix((mwSize)K, (mwSize)S, mxDOUBLE_CLASS, mxREAL);
+            mxArray* ge = gt ? mxCreateNumericMatrix((mwSize)K, (mwSize)S, mxDOUBLE_CLASS, mxREAL) : mxCreateNumericMatrix(0, 0, mxDOUBLE_CLASS, mxREAL);
+            if (!r && K) r = qmri_admm_history(st, (double*)mxGetData(dc), gt ? (double*)mxGetData(ge) : nullptr, &K);
+            qmri_admm_destroy(st);
+            if (r) {
+                mxDestroyArray(dc);
+                mxDestroyArray(ge);
+            }
+            check(r);
+            plhs[0] = x.finish();
+            const char* names[2] = {"dc_res", "gt_err"};
+            plhs[1] = mxCreateStructMatrix(1, 1, 2, names);
+            mxSetField(plhs[1], 0, "dc_res", dc);
+            mxSetField(plhs[1], 0, "gt_err", ge);
+        }
     } else if (cmd == "dict_load") {                         // (D single KxC, normD single, lut single KxQ) -> dict handle
         need(4);
         const mwSize* d = mxGetDimensions(prhs[1]);

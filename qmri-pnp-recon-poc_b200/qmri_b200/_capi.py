@@ -79,6 +79,8 @@ SIGNATURES = {
     "qmri_admm_destroy": (_i, [_vp]),
     "qmri_admm_xupdate_only": (_i, [_vp, _i]),
     "qmri_admm_xupdate_bytes": (_i, [_vp]),
+    "qmri_admm_monitor": (_i, [_vp, _i, _vp, _i]),
+    "qmri_admm_history": (_i, [_vp, _vp, _vp, C.POINTER(C.c_int)]),
     "qmri_dict_load": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _i, _i64, _i64, _pp]),
     "qmri_dict_load_shard": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _i, _i64, _i64, _pp]),
     "qmri_dict_destroy": (_i, [_vp]),

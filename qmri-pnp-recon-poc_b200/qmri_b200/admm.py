@@ -13,9 +13,17 @@ and returning ``N x M x 10`` (the pluggable proximal step of the reference; cost
 per iteration).  A trailing slice axis (``y: nmeas x S``, ``X0: N x M x C x S``) runs S
 independent reconstructions, each with its own min/max normalisation (``PnP_ADMM.m:121``).
 
-Differences from the reference, both deliberate: the least-squares step is solved exactly
-instead of by ``lsqr`` to ``cg_tol`` (identical to 1e-15 when ``A A^H = I``, SURVEY.md A.5),
-and the per-iteration progress prints (``:106-109``) are omitted.
+The least-squares step is solved exactly instead of by ``lsqr`` to ``cg_tol`` (identical to
+1e-15 when ``A A^H = I``, SURVEY.md A.5), a deliberate difference from the reference.
+
+The per-iteration progress of ``:106-109`` is not printed (that would stop the device loop
+once per iteration); ``x, info = PnP_ADMM(y, param, history=True)`` records it on the device
+instead and returns it after the run: ``info["dc_residual"]`` holds
+``|y - F.forward(x_k)| / |y|`` and ``info["gt_error"]`` ``|param.gt_tsmi - x_k| / |param.gt_tsmi|``
+(None without ``gt_tsmi``) for every iteration k, ``(iter, S)`` arrays (``(iter,)`` unbatched),
+with ``x_k`` the x-update output of iteration k, before the denoiser.  With ``history=False``
+``gt_tsmi`` is ignored and nothing extra runs.  :meth:`AdmmSession.monitor` /
+:meth:`AdmmSession.history` are the same on a resident session.
 """
 from __future__ import annotations
 
@@ -24,7 +32,7 @@ import ctypes as C
 import numpy as np
 
 from . import _capi
-from ._capi import AdmmParams, DENOISE_FN, as_f, check, dtype_code, ptr
+from ._capi import QMRI_EINVAL, AdmmParams, DENOISE_FN, QmriError, as_f, check, dtype_code, ptr
 from .denoiser import UNetRes
 from .operators import FOperator
 
@@ -98,7 +106,17 @@ def _prep_inputs(F, y, X0):
     return y, X0, S, batched
 
 
-def PnP_ADMM(y, param):
+def _prep_gt(F, gt, S):
+    gt = as_f(gt)
+    if gt.shape != (F.N, F.M, F.C, S) and not (S == 1 and gt.shape == (F.N, F.M, F.C)):
+        raise QmriError(QMRI_EINVAL, f"param.gt_tsmi must be {F.N} x {F.M} x {F.C}" + (f" x {S}" if S > 1 else "") +
+                        f", got {gt.shape}")
+    return gt
+
+
+def PnP_ADMM(y, param, history=False):
+    if history:
+        return _pnp_admm_history(y, param)
     keep = []
     p, F = _make_params(param, keep)
     y, X0, S, batched = _prep_inputs(F, y, param["X0"])
@@ -110,6 +128,25 @@ def PnP_ADMM(y, param):
             raise k
     check(rc)
     return x if batched else x[..., 0]
+
+
+def _pnp_admm_history(y, param):
+    X0 = param.get("X0")
+    batched = X0 is not None and np.ndim(X0) == 4
+    S = np.shape(X0)[3] if batched else 1
+    sess = AdmmSession(param, S)
+    try:
+        sess.monitor(param.get("gt_tsmi"))
+        sess.upload(y, X0)
+        sess.run()
+        x = sess.download()
+        info = sess.history()
+    finally:
+        sess.close()
+    if not batched:
+        x = x[..., 0]
+        info = {k: (None if v is None else v[:, 0]) for k, v in info.items()}
+    return x, info
 
 
 class AdmmSession:
@@ -124,6 +161,8 @@ class AdmmSession:
         h = C.c_void_p()
         check(self.lib.qmri_admm_create(self.F.P.handle, self.S, C.byref(self.p), C.byref(h)))
         self.handle = h
+        self._mon_gt = False     # a ground truth is attached (monitor)
+        self._run_gt = False     # ... and was for the last run (history)
 
     def upload(self, y, X0):
         y, X0, S, _ = _prep_inputs(self.F, y, X0)
@@ -135,7 +174,28 @@ class AdmmSession:
         """No host-side conversion: arrays must already be F-contiguous (pinned buffers welcome)."""
         check(self.lib.qmri_admm_upload(self.handle, ptr(y), dtype_code(y), ptr(X0), dtype_code(X0)))
 
+    def monitor(self, gt=None, enable=True):
+        """Record the convergence history of ``PnP_ADMM.m:106-109`` in every later run (see :meth:`history`).
+        ``gt``: the ground truth, ``N x M x C [x S]``, or None for the data-consistency residual only."""
+        if not enable:
+            check(self.lib.qmri_admm_monitor(self.handle, 0, None, 0))
+            self._mon_gt = False
+            return
+        g = None if gt is None else _prep_gt(self.F, gt, self.S)
+        check(self.lib.qmri_admm_monitor(self.handle, 1, ptr(g), 0 if g is None else dtype_code(g)))
+        self._mon_gt = g is not None
+
+    def history(self):
+        """History of the last run: ``{"dc_residual": (iters, S), "gt_error": (iters, S) or None}``, float64."""
+        n = C.c_int()
+        check(self.lib.qmri_admm_history(self.handle, None, None, C.byref(n)))
+        dc = np.zeros((n.value, self.S), np.float64, order="F")
+        gt = np.zeros((n.value, self.S), np.float64, order="F") if self._run_gt else None
+        check(self.lib.qmri_admm_history(self.handle, ptr(dc), ptr(gt), C.byref(n)))
+        return {"dc_residual": dc, "gt_error": gt}
+
     def run(self, iters=None):
+        self._run_gt = self._mon_gt
         check(self.lib.qmri_admm_run(self.handle, int(self.p.iters if iters is None else iters)))
         for k in self._keep:
             if isinstance(k, Exception):
