@@ -1,4 +1,4 @@
-"""The benchmark job at 256 x 256: 8 volunteers x 15 slices from benchdata.make_qmaps(N=256, M=256), TSMIs synthesised on the
+"""The benchmark job at N x N (--side, default 256): 8 volunteers x 15 slices from benchdata.make_qmaps(N=N, M=N), TSMIs synthesised on the
 device, 30 dB AWGN, spiral mask (S = 771), rho = 0.05, 100 PnP-ADMM iterations with the random-init UNetRes (tensor mode), then
 matching against 100 000 atoms - timed like bench.py (DESIGN.md section 5: CUDA events on the library's stream, warm-up first,
 a 256 MiB buffer written between steps so the 1.6 GB of loop state is not served from L2).
@@ -6,7 +6,7 @@ a 256 MiB buffer written between steps so the 1.6 GB of loop state is not served
 Prints one JSON line (and writes it to --out): slice-iterations/s of the job, the x-update alone (us per slice-iteration and its
 fraction of HBM counted at 20 B per pixel-channel), ms per denoiser forward, single-slice reconstruction latency, and the GPU's
 name and power limit read in the same run.
-Usage (GPU box): python profiles/tools/job256.py [--steps 2] [--warmup 1] [--out FILE]"""
+Usage (GPU box): python profiles/tools/job256.py [--side 256] [--steps 2] [--warmup 1] [--out FILE]"""
 import argparse
 import ctypes as C
 import json
@@ -38,8 +38,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=1)
     ap.add_argument("--iters", type=int, default=100)
     ap.add_argument("--atoms", type=int, default=100000)
+    ap.add_argument("--side", type=int, default=256, help="image side N == M (160, 192, 224 or 256)")
     ap.add_argument("--out")
     args = ap.parse_args()
+    global N, HW
+    N, HW = args.side, args.side * args.side
     import torch
     import bench
     import benchdata
@@ -58,7 +61,7 @@ def main():
     d = q.Dictionary(dct, ctx=ctx)
     X = np.empty((N, N, C_CH, S), np.float64, order="F")
     for vol in range(VOLUNTEERS):
-        qm = benchdata.make_qmaps(seed=vol, S=PER_VOLUNTEER, N=N, M=N)              # [15 x 3 x 256 x 256]
+        qm = benchdata.make_qmaps(seed=vol, S=PER_VOLUNTEER, N=N, M=N)              # [15 x 3 x N x N]
         for sl in range(PER_VOLUNTEER):
             X[..., vol * PER_VOLUNTEER + sl] = q.synthesize_tsmis(d, qm[sl])          # on the GPU
     P = q.setup_subsampling_spiralgrided(N, N, bench.SPIRAL_S, np.eye(C_CH), ctx=ctx)
@@ -142,7 +145,7 @@ def main():
     sess1.close()
 
     line = {
-        "what": f"256 x 256 job: {S}-slice PnP-ADMM recon (spiral S = {bench.SPIRAL_S}, {P.nmeas // C_CH} samples per frame, rho {bench.RHO}, "
+        "what": f"{N} x {N} job: {S}-slice PnP-ADMM recon (spiral S = {bench.SPIRAL_S}, {P.nmeas // C_CH} samples per frame, rho {bench.RHO}, "
                 f"{iters} iterations, random-init UNetRes 10->10 in tensor mode) + matching ({d.K} atoms, cut3)",
         "gpu": info,
         "slice_iterations_per_s": S * iters * args.steps / (ms_job * 1e-3),

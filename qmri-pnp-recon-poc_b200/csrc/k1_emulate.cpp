@@ -420,11 +420,11 @@ int k1emu_run(int mode, int mc, int pattern, double arg, int C, int S, const flo
     return t.nmeas;
 }
 
-// The streaming kernels at image side n (224 or 256; N == M), same modes and arguments as k1emu_run.  Returns nmeas, -1 if the
-// mask does not fit the work-item tables, -2 for another side.
+// The streaming kernels at image side n (160, 192, 224 or 256; N == M), same modes and arguments as k1emu_run.  Returns nmeas, -1 if
+// the mask does not fit the work-item tables, -2 for another side.
 int k1emu_run_n(int n, int mode, int pattern, double arg, int C, int S, const float* in_re, const float* in_im, const float* v,
                 const float* y, float rho, float* out_re, float* out_im, float* y_out, float* minmax) {
-    if (n != 224 && n != 256) return -2;
+    if (n != 160 && n != 192 && n != 224 && n != 256) return -2;
     std::vector<std::vector<int32_t>> frames;
     if (pattern == 0) optab::spiral_frames(n, (int)arg, C, frames);
     else optab::epi_frames(n, n, arg, C, frames);
@@ -432,8 +432,12 @@ int k1emu_run_n(int n, int mode, int pattern, double arg, int C, int S, const fl
     const char* env = getenv("QMRI_K1_QMIN");
     optab::build_k1_tables(n, frames, t, env ? atoi(env) : 8);
     if (!t.stream_ok) return -1;
-    if (n == 224) emulate_stream<224>(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax);
-    else emulate_stream<256>(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax);
+    switch (n) {
+        case 160: emulate_stream<160>(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax); break;
+        case 192: emulate_stream<192>(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax); break;
+        case 224: emulate_stream<224>(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax); break;
+        default: emulate_stream<256>(mode, C, S, t, in_re, in_im, v, y, rho, out_re, out_im, y_out, minmax);
+    }
     return t.nmeas;
 }
 

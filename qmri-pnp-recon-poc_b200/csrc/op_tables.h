@@ -93,7 +93,7 @@ struct K1Tables {
     std::vector<uint16_t> r_rowmask;  // [C][16] like rowmask, symmetric: row k and row N - k are set together
     int r_n_ovf = 0;
     std::vector<float> tw2;           // [16][16][2]  e^{-2 pi i (i j) / N}
-    std::vector<float> tw448;         // [2N][2]      e^{-2 pi i t / (2N)} (448 entries at N = 224, 512 at N = 256)
+    std::vector<float> tw448;         // [2N][2]      e^{-2 pi i t / (2N)} (320, 384, 448 or 512 entries at N = 160, 192, 224, 256)
 };
 
 constexpr int K1_PHASES = 8;          // row phases of the sparse inverse pass = THREADS / MC of the kernel
@@ -106,7 +106,7 @@ static inline uint32_t p4_entry(int k2, int k1, int j, bool last) {
 constexpr int STREAM_QMAX = 64;      // == k1::QMAX_STREAM
 constexpr int STREAM_OVF_MAX = 96;   // == k1::OVF_MAX_STREAM
 
-// Work items of the streaming kernel (N = 224 or 256 threads, one per k-space row).  Every item carries at least one sample, so
+// Work items of the streaming kernel (N = 160, 192, 224 or 256 threads, one per k-space row).  Every item carries at least one sample, so
 // cnt == 0 marks a thread without an item (k1 takes all 8 bits: row 255 is a real row at N = 256).
 // The samples of a k-space row k1 are cut into chunks of at most Q samples (Q = the
 // smallest value for which the frame needs no more than N items, so a thread never carries more than one); the row's first
@@ -179,7 +179,7 @@ static inline bool stream_items_for_frame(int N, const std::vector<std::vector<u
 }
 
 static inline void build_stream_tables(int N, const std::vector<std::vector<int32_t>>& frames, K1Tables& t, int q_min = 1) {
-    t.stream_ok = N == 224 || N == 256;  // the sides the streaming kernels are instantiated for
+    t.stream_ok = N == 160 || N == 192 || N == 224 || N == 256;  // the sides the streaming kernels are instantiated for
     t.itA.assign((size_t)t.C * N, 255u);
     t.itB.assign((size_t)t.C * N, 0u);
     t.ent.assign(std::max(t.nmeas, 1), 0);

@@ -338,8 +338,8 @@ struct qmri_op {
 static int op_from_frames(qmri_ctx* ctx, int N, int M, int C, int L, const std::vector<std::vector<int32_t>>& frames,
                           const double* V, qmri_op** out) {
     if (!ctx || !out) return qmri_fail(QMRI_EINVAL, "operator: null argument");
-    if (N != M || (N != 224 && N != 256))
-        return qmri_fail(QMRI_EUNSUPPORTED, "this build supports N == M == 224 or 256 (got %d x %d)", N, M);
+    if (N != M || (N != 160 && N != 192 && N != 224 && N != 256))
+        return qmri_fail(QMRI_EUNSUPPORTED, "this build supports N == M == 160, 192, 224 or 256 (got %d x %d)", N, M);
     if (C < 1 || C > 64) return qmri_fail(QMRI_EINVAL, "C = %d out of range", C);
     bool identity = (L == C);
     if (V && identity) {
@@ -372,11 +372,11 @@ static int op_from_frames(qmri_ctx* ctx, int N, int M, int C, int L, const std::
     env = getenv("QMRI_K1_QMIN");  // tuning knob: smallest chunk size tried for the streaming kernel's work items
     const int q_min = env ? atoi(env) : 8;  // 8: measured best on the spiral masks (fewer overflow partials)
     optab::build_k1_tables(N, frames, op->t, q_min);
-    if (N == 256 && identity && !op->t.stream_ok) {  // 256: the streaming kernels are the only x-update kernels
+    if (N != 224 && identity && !op->t.stream_ok) {  // sides other than 224: the streaming kernels are the only x-update kernels
         const int max_row = op->t.max_row;
         delete op;
-        return qmri_fail(QMRI_EUNSUPPORTED, "N == M == 256: the mask does not fit the streaming kernel's work-item tables (densest k-space "
-                         "row: %d samples)", max_row);
+        return qmri_fail(QMRI_EUNSUPPORTED, "N == M == %d: the mask does not fit the streaming kernel's work-item tables (densest k-space "
+                         "row: %d samples)", N, max_row);
     }
     op->general = !identity;
     if (!identity) op->hV.assign(V, V + (size_t)L * C);
@@ -507,7 +507,7 @@ extern "C" int qmri_op_indices(const qmri_op* op, int32_t* idx, int64_t* frame_p
 // per slice-channel image) from about two slices on, the single cluster kernel (xupdate_kernel.cu: the image stays in the
 // shared memory of eight CTAs) below that - measured on B200: 23.8 vs 27.0 us at one slice, 16.2 vs 15.5 us at two, 9.1 vs
 // 7.4 us at eight, 6.97 vs 4.13 us per slice at 120.  QMRI_K1_KERNEL=cluster|stream forces one (tests, profiling).
-// N == M == 256: the cluster kernel is built for 224 only, so the streaming kernels run at every batch size.
+// N == M != 224 (160, 192, 256): the cluster kernel is built for 224 only, so the streaming kernels run at every batch size.
 // part / cbuf: scratch of the streaming kernels.  The host entry points use the operator's; an ADMM session brings its own,
 // sized once for its batch, because its CUDA graph keeps the addresses.
 // General V: forward transform of every channel on the union mask (one launch per part of the union) -> per-location channel
@@ -626,11 +626,11 @@ static int k1_dispatch(qmri_op* op, const K1Params& p_in, int S, DevBuf* part = 
     qmri_ctx* ctx = op->ctx;
     const bool can_stream = op->t.stream_ok;
     bool stream = can_stream && (long long)S * op->C * K1_STREAM_MIN_IMAGES_DIV >= (long long)ctx->sm_count;
-    if (op->N == 256 || monitored) {
-        if (op->k1_kernel == 1 && op->N == 256)
+    if (op->N != 224 || monitored) {
+        if (op->k1_kernel == 1 && op->N != 224)
             return qmri_fail(QMRI_EUNSUPPORTED, "QMRI_K1_KERNEL=cluster: the cluster x-update kernel supports N == M == 224 only (operator is "
                              "%d x %d)", op->N, op->M);
-        stream = true;  // stream_ok: checked when the operator was built (256) or by k1_monitor_supported
+        stream = true;  // stream_ok: checked when the operator was built (N != 224) or by k1_monitor_supported
     }
     if (op->k1_kernel == 1) stream = false;
     if (op->k1_kernel == 2) {

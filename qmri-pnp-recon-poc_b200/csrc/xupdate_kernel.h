@@ -30,7 +30,7 @@ struct K1Params {
     int p4_len;
     // streaming kernel tables (xupdate_stream.cu; op_tables.h)
     const float2* tw2;       // [16][16] e^{-2 pi i (i j) / N}
-    const float2* tw448;     // [2N] e^{-2 pi i t / (2N)} (448 entries at N = 224, 512 at N = 256)
+    const float2* tw448;     // [2N] e^{-2 pi i t / (2N)} (2N entries)
     const uint32_t* itA;     // [C][N] work item of thread tid: k1 | cnt << 8 | start << 16 (cnt == 0: no item)
     const uint32_t* itB;     // [C][N] slot | novf << 8 | ovf0 << 16
     const uint32_t* ent;     // [nmeas] j | k2 << 16, frame-major, grouped by item
@@ -50,7 +50,7 @@ struct K1Params {
     int mode;
     float inv_1p_rho;
     double rho;              // host side only (general V: selects the precomputed (G_k + rho I)^{-1})
-    int nf;                  // image side N == M: 224 (every kernel) or 256 (streaming kernels only)
+    int nf;                  // image side N == M: 224 (every kernel) or 160, 192, 256 (streaming kernels only)
     // PnP-ADMM progress monitor (qmri_admm_monitor; streaming kernels, modes ADMM and SOLVE): the monitored kernel instances write
     // double partial sums, each reduced in a fixed order.  Null: the unmonitored instances run.
     double* mon_dc;          // [S][C] sum over the channel's samples of |y - A z|^2 (stream_solve_kernel; general V: GeneralMix)
@@ -61,7 +61,7 @@ struct K1Params {
 
 int k1_launch(qmri_ctx* ctx, const K1Params& p, int S, int ns_max, int mc);  // cluster kernel: N == M == 224 only
 constexpr int K1_STREAM_MIN_IMAGES_DIV = 8;  // streaming kernels from S * C >= SM count / 8 images on (two 10-channel slices on B200)
-// streaming variant: G CTAs per (slice, channel); needs K1Tables::stream_ok.  The only x-update kernels for N == 256.
+// streaming variant: G CTAs per (slice, channel); needs K1Tables::stream_ok.  The only x-update kernels for N != 224.
 int k1_stream_groups(int S, int C, int sm_count);
 size_t k1_stream_part_elems(int S, int C, int G, int ns_max);
 size_t k1_stream_cbuf_elems(int S, int C, int ns_max);

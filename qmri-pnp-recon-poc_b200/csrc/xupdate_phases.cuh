@@ -10,7 +10,7 @@
 // A^H c is the inverse transform of a sparse array, so the m-direction transforms
 // are evaluated as sparse DFT sums, and only the n-direction (contiguous dim) uses
 // full length-224 FFTs (224 = 14 x 16, two register-resident stages).  The streaming kernels
-// (xupdate_stream.cu) also run N == M == 256 = 16 x 16: see Side below.
+// (xupdate_stream.cu) also run N == M == 160 = 10 x 16, 192 = 12 x 16 and 256 = 16 x 16: see Side below.
 //
 // The functions here are __host__ __device__ so that tests/test_k1_emulation.py can
 // run the exact kernel arithmetic on the CPU (no GPU in the build container).
@@ -103,6 +103,94 @@ QHD void dft4(float2& a, float2& b, float2& c, float2& d) {
     d = csub(s1, s3);
 }
 
+// ---- 5-point DFT (forward, e^{-2 pi i/5}) ----------------------------------------
+QHD void dft5(float2& x0, float2& x1, float2& x2, float2& x3, float2& x4) {
+    const float C1 = 0.30901699437494742f, C2 = -0.80901699437494742f;
+    const float S1 = 0.95105651629515357f, S2 = 0.58778525229247313f;
+    float2 p1 = cadd(x1, x4), p2 = cadd(x2, x3);
+    float2 q1 = csub(x1, x4), q2 = csub(x2, x3);
+    float2 a1 = make_float2(x0.x + C1 * p1.x + C2 * p2.x, x0.y + C1 * p1.y + C2 * p2.y);
+    float2 a2 = make_float2(x0.x + C2 * p1.x + C1 * p2.x, x0.y + C2 * p1.y + C1 * p2.y);
+    float2 b1 = make_float2(S1 * q1.x + S2 * q2.x, S1 * q1.y + S2 * q2.y);
+    float2 b2 = make_float2(S2 * q1.x - S1 * q2.x, S2 * q1.y - S1 * q2.y);
+    x0 = make_float2(x0.x + p1.x + p2.x, x0.y + p1.y + p2.y);
+    // X_k = A_k - i B_k ; X_{5-k} = A_k + i B_k
+    x1 = make_float2(a1.x + b1.y, a1.y - b1.x);
+    x4 = make_float2(a1.x - b1.y, a1.y + b1.x);
+    x2 = make_float2(a2.x + b2.y, a2.y - b2.x);
+    x3 = make_float2(a2.x - b2.y, a2.y + b2.x);
+}
+
+// e^{-2 pi i k / 10}, k = 0..4
+QHD float2 w10(int k) {
+    switch (k) {
+        case 0: return make_float2(1.0f, 0.0f);
+        case 1: return make_float2(0.80901699437494742f, -0.58778525229247313f);
+        case 2: return make_float2(0.30901699437494742f, -0.95105651629515357f);
+        case 3: return make_float2(-0.30901699437494742f, -0.95105651629515357f);
+        default: return make_float2(-0.80901699437494742f, -0.58778525229247313f);
+    }
+}
+
+// 10-point DFT, natural order in and out (radix-2 DIT over two 5-point DFTs)
+QHD void dft10(float2 (&x)[16]) {
+    float2 e0 = x[0], e1 = x[2], e2 = x[4], e3 = x[6], e4 = x[8];
+    float2 o0 = x[1], o1 = x[3], o2 = x[5], o3 = x[7], o4 = x[9];
+    dft5(e0, e1, e2, e3, e4);
+    dft5(o0, o1, o2, o3, o4);
+    float2 t;
+    x[0] = cadd(e0, o0); x[5] = csub(e0, o0);
+    t = cmul(o1, w10(1)); x[1] = cadd(e1, t); x[6] = csub(e1, t);
+    t = cmul(o2, w10(2)); x[2] = cadd(e2, t); x[7] = csub(e2, t);
+    t = cmul(o3, w10(3)); x[3] = cadd(e3, t); x[8] = csub(e3, t);
+    t = cmul(o4, w10(4)); x[4] = cadd(e4, t); x[9] = csub(e4, t);
+}
+
+// ---- 3-point DFT (forward, e^{-2 pi i/3}) ----------------------------------------
+QHD void dft3(float2& x0, float2& x1, float2& x2) {
+    const float S = 0.86602540378443865f;
+    const float2 p = cadd(x1, x2), q = csub(x1, x2);
+    const float2 a = make_float2(x0.x - 0.5f * p.x, x0.y - 0.5f * p.y);
+    const float2 b = make_float2(S * q.x, S * q.y);
+    x0 = cadd(x0, p);
+    // X_1 = A - i B ; X_2 = A + i B
+    x1 = make_float2(a.x + b.y, a.y - b.x);
+    x2 = make_float2(a.x - b.y, a.y + b.x);
+}
+
+// e^{-2 pi i k / 12}, k = 1, 2, 4 (the twiddles of 3x4 other than -i and -1)
+QHD float2 w12(int k) {
+    const float h = 0.86602540378443865f;
+    switch (k) {
+        case 1: return make_float2(h, -0.5f);
+        case 2: return make_float2(0.5f, -h);
+        default: return make_float2(-0.5f, -h);  // k == 4
+    }
+}
+
+// 12-point DFT, natural order in and out: n = 4a + b (a < 3, b < 4), k = ka + 3 kb
+QHD void dft12(float2 (&x)[16]) {
+#pragma unroll
+    for (int b = 0; b < 4; ++b) dft3(x[b], x[4 + b], x[8 + b]);  // over a; result index ka at x[4 ka + b]
+    // twiddles w12^{ka b}: exponents 1, 2, 3 (ka = 1) and 2, 4, 6 (ka = 2); 3 is -i, 6 is -1
+    x[5] = cmul(x[5], w12(1));
+    x[6] = cmul(x[6], w12(2));
+    x[7] = mul_mi(x[7]);
+    x[9] = cmul(x[9], w12(2));
+    x[10] = cmul(x[10], w12(4));
+    x[11] = make_float2(-x[11].x, -x[11].y);
+#pragma unroll
+    for (int ka = 0; ka < 3; ++ka) dft4(x[4 * ka + 0], x[4 * ka + 1], x[4 * ka + 2], x[4 * ka + 3]);  // over b; kb at x[4 ka + kb]
+    // x[4 ka + kb] holds X[ka + 3 kb] -> natural order
+    float2 t[12];
+#pragma unroll
+    for (int i = 0; i < 12; ++i) t[i] = x[i];
+#pragma unroll
+    for (int ka = 0; ka < 3; ++ka)
+#pragma unroll
+        for (int kb = 0; kb < 4; ++kb) x[ka + 3 * kb] = t[4 * ka + kb];
+}
+
 // e^{-2 pi i k / 16}, k = 0..9 (all that 4x4 needs)
 QHD float2 w16(int k) {
     const float c1 = 0.92387953251128674f, s1 = 0.38268343236508977f, r = 0.70710678118654752f;
@@ -152,7 +240,8 @@ QHD void fft_s1_load(const float2* col, int n2, const float2* tw, float2 (&a)[16
 #pragma unroll
     for (int k1 = 1; k1 < 14; ++k1) a[k1] = cmul(a[k1], tw[n2 * k1]);
 }
-// (the stage-1 store and the stage-2 store / loads below are shared with the streaming kernels, which also run N = 256: R = N / 16)
+// (the stage-1 store and the stage-2 store / loads below are shared with the streaming kernels, which also run N = 160, 192 and 256:
+// R = N / 16)
 template <int N = NF>
 QHD void fft_s1_store(float2* col, int n2, const float2 (&a)[16]) {
 #pragma unroll
@@ -217,8 +306,9 @@ QHD void sparse_idft_flat(float2* col, const float2* c, const float2* twp, const
 // =====================================================================================
 // Streaming variant (xupdate_stream.cu): one CTA walks the sixteen R-column slabs of a
 // (slice, channel) image one after the other, so no cluster exchange is needed.
-// Image sides N = 16 R: 224 (R = 14) and 256 (R = 16); the functions below take N as a template
-// argument, and the 224 instance is the arithmetic of the original 224-only kernels.
+// Image sides N = 16 R: 160 (R = 10), 192 (R = 12), 224 (R = 14) and 256 (R = 16); the functions below take N as a template
+// argument, and the 224 instance is the arithmetic of the original 224-only kernels.  R is even at every side, so the NP = R / 2
+// column pairs of the sparse sums cover the slab.
 //  * the first forward stage takes its R inputs from registers (loaded straight from
 //    global memory), the last inverse stage leaves its R outputs in registers (stored
 //    straight to global memory): two shared-memory passes fewer per transform;
@@ -231,7 +321,7 @@ QHD void sparse_idft_flat(float2* col, const float2* c, const float2* twp, const
 // =====================================================================================
 template <int N>
 struct Side {
-    static_assert(N == 224 || N == 256, "streaming kernels: N == M == 224 or 256");
+    static_assert(N == 160 || N == 192 || N == 224 || N == 256, "streaming kernels: N == M == 160, 192, 224 or 256");
     static constexpr int R = N / 16;            // radix of the first forward / last inverse stage = columns per slab
     static constexpr int CS = N + 1;            // shared-memory column stride in float2 (odd: conflict-free across columns)
     static constexpr int NP = R / 2;            // column pairs per slab in the sparse sums
@@ -239,7 +329,9 @@ struct Side {
 };
 template <int R>
 QHD void dft_r(float2 (&x)[16]) {
-    if constexpr (R == 14) dft14(x);
+    if constexpr (R == 10) dft10(x);
+    else if constexpr (R == 12) dft12(x);
+    else if constexpr (R == 14) dft14(x);
     else dft16(x);
 }
 
@@ -300,7 +392,7 @@ QHD void inv_s2_regs(const float2* col, int c, float2 (&x)[16]) {
 // (d = d' + 1/2):
 //   e^{-i phi (base +- d)} = tc * r_d^{+-1},   tc = e^{-i phi base} (base = m0 + NP - 1/2),   r_d = e^{-i phi d},   phi = 2 pi k2 / N
 // so with P_d = T[NP+d'] + T[NP-1-d'], M_d = T[NP+d'] - T[NP-1-d'] (formed once per item) a sample costs 4 FMAs and one twiddle
-// rotation per column PAIR.  tw2n[x] = e^{-2 pi i x / (2N)} (448 or 512 entries; K1Params::tw448) supplies the half-integer phases.
+// rotation per column PAIR.  tw2n[x] = e^{-2 pi i x / (2N)} (2N entries; K1Params::tw448) supplies the half-integer phases.
 constexpr int HC_STREAM = Side<NF>::R;
 constexpr int NP_STREAM = Side<NF>::NP;          // column pairs per half slab of the real-image kernels
 constexpr int OVF_STRIDE = Side<NF>::OVF_STRIDE;

@@ -15,8 +15,9 @@
 //   stream_solve_kernel   grid (C, S): adds the G partials in a fixed order, c = (y - A z) / (1 + rho)
 //   stream_adj_kernel     grid (G, C, S): sparse inverse DFT along m -> inverse FFT along n -> registers ->
 //                         w' = v + corr (+ x on the last iteration) -> global; per-slice min / max
-// Two instances of each kernel, by image side N == M: 224 (R = 14: CTAs of 224 threads, four per SM) and 256 (R = 16: CTAs of
-// 256 threads, three per SM for the forward kernel and two for the adjoint kernel - see fwd_min_ctas / adj_min_ctas).
+// One instance of each kernel per image side N == M = 16 R, with CTAs of N threads: 224 (R = 14, four CTAs per SM), 256 (R = 16,
+// three per SM for the forward kernel and two for the adjoint kernel), 160 (R = 10) and 192 (R = 12) - see fwd_min_ctas /
+// adj_min_ctas.
 // No cluster, no DSMEM, work items small enough that the last wave is short.  The first / last FFT stage works on registers filled from / drained to global memory and the
 // sparse sums run on per-row work items with rotating twiddles (xupdate_phases.cuh), so the shared-memory
 // traffic is about a third of the cluster kernel's.  HBM traffic per pixel-channel: read w (8 B) + v (4 B)
@@ -36,12 +37,18 @@ namespace {
 // Per image side N: R = N / 16 columns per slab, N threads = R column FFTs x 16 lanes (in the sparse passes one thread per work
 // item, i.e. per k-space row), 16 slabs per image.
 constexpr int SLABS = 16;
-// CTAs per SM the register allocation is fitted to.  N = 256: the forward kernel fits three (80 registers); the adjoint kernel
-// needs more than 80 (at three it spills the work-item fields it keeps across the slab loop), so it is fitted to two.
+// CTAs per SM the register allocation is fitted to (ptxas -v, sm_100a; a CTA's warps are spread over the SM's four register-file
+// quarters, so k CTAs of w warps leave 16384 / (32 ceil(k w / 4)) registers per thread).
+//  * N = 256: the forward kernel fits three (80 registers); the adjoint kernel needs more than 80 (at three it spills the work-item
+//    fields it keeps across the slab loop), so it is fitted to two.
+//  * N = 192: the forward kernel fits five (63 registers).  The adjoint kernel spills 4 - 8 bytes at three (96 registers), so it is
+//    fitted to two (166 - 168 registers, no spills).
+//  * N = 160: the forward kernel fits six (63 - 64 registers).  The adjoint kernel spills 60 - 72 bytes at five (72 registers) and
+//    28 bytes at four (96 registers, all modes but ADMM), so it is fitted to three (128 registers, no spills).
 template <int N>
-constexpr int fwd_min_ctas() { return N == 224 ? 4 : 3; }
+constexpr int fwd_min_ctas() { return N == 160 ? 6 : N == 192 ? 5 : N == 224 ? 4 : 3; }
 template <int N>
-constexpr int adj_min_ctas() { return N == 224 ? 4 : 2; }
+constexpr int adj_min_ctas() { return N == 160 ? 3 : N == 192 ? 2 : N == 224 ? 4 : 2; }
 // The monitored SOLVE instance (the first x-update of a monitored PnP-ADMM run, once per run) is fitted to one CTA less at 224:
 // at four its ground-truth loads add spills.
 template <int N, int MODE, bool MON>
@@ -442,7 +449,11 @@ int k1_stream_launch(qmri_ctx* ctx, const K1Params& p_in, int S, int ns_max) {
         p.slot_off = 0;
         p.slot_stride = ns_max;
     }
-    if (p.nf == 224) return launch_side<224>(ctx, p, S);
-    if (p.nf == 256) return launch_side<256>(ctx, p, S);
-    return qmri_fail(QMRI_EUNSUPPORTED, "x-update (streaming kernel): image side %d (224 or 256)", p.nf);
+    switch (p.nf) {
+        case 160: return launch_side<160>(ctx, p, S);
+        case 192: return launch_side<192>(ctx, p, S);
+        case 224: return launch_side<224>(ctx, p, S);
+        case 256: return launch_side<256>(ctx, p, S);
+    }
+    return qmri_fail(QMRI_EUNSUPPORTED, "x-update (streaming kernel): image side %d (160, 192, 224 or 256)", p.nf);
 }
