@@ -243,6 +243,38 @@ int qmri_match_finish_dev(qmri_dict* d, const float* x_re, const float* x_im, in
  * atom_index (optional): 1-based I.  Exact distance ties resolve to the lowest atom index. */
 int qmri_synthesize(qmri_dict* d, const float* qmap, int64_t npix, float* X, int32_t* atom_index);
 
+/* ---- FISP-MRF dictionary simulation ---------------------------------------------------
+ * Builds the dict struct the reference loads at main_recon_tsmis_FFT.m:127-129 and main_synthesize_tsmis.m:50-54
+ * (dictionaries/real_fisp_cut*_dict/SVD_dict_FISP_cut*.mat; fields as in mrf_dtm_cpu.m:8-12), cut = the first T pulses
+ * (main_recon_tsmis_FFT.m:42: T = 1000, 500, 300, 200, 100).
+ * Signal model: FISP with one full dephasing cycle per TR, RF phase 0, ideal pulses, B1 = 1, no off-resonance, extended phase
+ * graph with Weigel's operators.  Start Z0 = 1, or 1 - 2 exp(-ti/T1) after an ideal inversion ti seconds before pulse 0; per
+ * pulse i: rotation T(flip_deg[i], 0) on every order, sample d_i = i F+_0 exp(-te/T2) (real), relaxation over tr[i]
+ * (F *= E2, Z *= E1, Z0 += 1 - E1), shift by one order.  Computed in fp32; the Gram matrix in double.
+ * Limits: 1 <= T <= 1024 (longer schedules: QMRI_EUNSUPPORTED), 1 <= C <= min(T, 16), K < 2^32.  QMRI_EINVAL for null pointers,
+ * non-finite or negative flip angles, tr <= 0, te outside [0, min tr], ti < 0, T1 or T2 <= 0 or non-finite, an empty or
+ * out-of-range atom range. */
+typedef struct qmri_fisp_seq {
+    int T;                  /* pulses = time points (cut0..cut4: 1000, 500, 300, 200, 100) */
+    const double* flip_deg; /* T flip angles in degrees, RF phase 0                       */
+    const double* tr;       /* T repetition times in seconds                              */
+    double te;              /* echo time in seconds                                       */
+    int inversion;          /* 1: ideal inversion ti seconds before pulse 0               */
+    double ti;
+} qmri_fisp_seq;
+/* lut: K x 2 column-major float32 (T1, T2 in seconds) - the dict.lut the outputs belong to.  The atoms simulated are exactly
+ * these float32 values. */
+/* Raw fingerprints, sig: K x T column-major. */
+int qmri_fisp_signals(qmri_ctx* ctx, const qmri_fisp_seq* seq, const float* lut, int64_t K, float* sig);
+/* Temporal Gram matrix G = sum_k d_k d_k^T (T x T, exactly symmetric; products exact in double, summed in a fixed order: the same
+ * inputs give the same bits).  Its top-C eigenvectors are dict.V; the eigen-decomposition is the caller's (numpy.linalg.eigh,
+ * MATLAB eig). */
+int qmri_fisp_gram(qmri_ctx* ctx, const qmri_fisp_seq* seq, const float* lut, int64_t K, double* G);
+/* Atoms [atom_begin, atom_end) projected onto V (T x C column-major):  D = d V / |d V| ((end-begin) x C column-major float32)
+ * and normD = |d V| (end-begin floats).  No K x T array is formed; an atom's row does not depend on the range it is built in. */
+int qmri_fisp_compress(qmri_ctx* ctx, const qmri_fisp_seq* seq, const float* lut, int64_t K, const double* V, int C,
+                       int64_t atom_begin, int64_t atom_end, float* D, float* normD);
+
 /* ---- foreground mask and quality metrics (SURVEY.md 8f-4) ------------------------------
  * mask = getmask_fromPD(PD, thresh)   main_files/utils/getmask_fromPD.m:1-15 (called at main_recon_tsmis_FFT.m:190):
  * |PD| / max, values below thresh zeroed, holes filled (8-connected background), binarised.  pd: N x M column-major,

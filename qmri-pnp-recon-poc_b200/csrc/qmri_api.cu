@@ -6,11 +6,13 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <vector>
 
 #include "aux_kernels.h"
 #include "common.cuh"
 #include "conv_kernels.h"
+#include "fisp_kernels.h"
 #include "lrtv_kernels.h"
 #include "match_kernel.h"
 #include "op_tables.h"
@@ -1654,6 +1656,146 @@ extern "C" int qmri_synthesize(qmri_dict* d, const float* qmap, int64_t npix, fl
     QCHECK(k4_launch(ctx, p));
     QCUDA(cudaMemcpyAsync(X, p.X, n * d->C * 4, cudaMemcpyDeviceToHost, ctx->stream));
     if (atom_index) QCUDA(cudaMemcpyAsync(atom_index, p.index, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    QCUDA(cudaStreamSynchronize(ctx->stream));
+    return QMRI_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// FISP-MRF dictionary simulation (dict.{D, normD, lut, V}, main_recon_tsmis_FFT.m:127-129)
+// ------------------------------------------------------------------------------------------
+// Atoms per simulated chunk of raw fingerprints (qmri_fisp_signals, qmri_fisp_gram): 128 MB of scratch at T = 1024, for any K.
+constexpr int64_t FISP_CHUNK = 32768;
+
+// Device copies of one call's schedule and look-up table; everything is freed when the call returns.
+struct FispCall {
+    qmri_ctx* ctx;
+    DevBuf pulse, tr, lut, V, out, aux, part, G;
+    FispParams p;
+    explicit FispCall(qmri_ctx* c) : ctx(c) {}
+    ~FispCall() {
+        cudaStreamSynchronize(ctx->stream);
+        for (DevBuf* b : {&pulse, &tr, &lut, &V, &out, &aux, &part, &G}) b->release();
+    }
+};
+
+static int fisp_begin(FispCall& w, const qmri_fisp_seq* seq, const float* lut, int64_t K, const char* fn) {
+    if (!seq || !lut || !seq->flip_deg || !seq->tr) return qmri_fail(QMRI_EINVAL, "%s: null argument", fn);
+    const int T = seq->T;
+    if (T < 1) return qmri_fail(QMRI_EINVAL, "%s: T = %d pulses", fn, T);
+    if (T > FISP_MAX_T) return qmri_fail(QMRI_EUNSUPPORTED, "%s: T = %d pulses; this build simulates at most %d", fn, T, FISP_MAX_T);
+    if (K < 1 || K >= 0xFFFFFFFFll) return qmri_fail(QMRI_EINVAL, "%s: K = %lld atoms out of range", fn, (long long)K);
+    double tr_min = INFINITY;
+    std::vector<float4> pulse(T);
+    std::vector<float> tr(T);
+    for (int i = 0; i < T; ++i) {
+        const double a = seq->flip_deg[i], t = seq->tr[i];
+        if (!std::isfinite(a) || a < 0.0) return qmri_fail(QMRI_EINVAL, "%s: flip_deg[%d] = %g must be finite and >= 0", fn, i, a);
+        if (!std::isfinite(t) || !(t > 0.0)) return qmri_fail(QMRI_EINVAL, "%s: tr[%d] = %g must be finite and > 0", fn, i, t);
+        tr_min = std::min(tr_min, t);
+        const double r = a * M_PI / 180.0, c = cos(0.5 * r), s = sin(0.5 * r);
+        pulse[i] = make_float4((float)(c * c), (float)(s * s), (float)sin(r), (float)cos(r));
+        tr[i] = (float)t;
+    }
+    if (!(seq->te >= 0.0) || seq->te > tr_min) return qmri_fail(QMRI_EINVAL, "%s: te = %g outside [0, min tr = %g]", fn, seq->te, tr_min);
+    if (seq->inversion != 0 && seq->inversion != 1) return qmri_fail(QMRI_EINVAL, "%s: inversion must be 0 or 1", fn);
+    if (seq->inversion && !(std::isfinite(seq->ti) && seq->ti >= 0.0)) return qmri_fail(QMRI_EINVAL, "%s: ti = %g must be finite and >= 0", fn, seq->ti);
+    for (int64_t k = 0; k < 2 * K; ++k)
+        if (!std::isfinite(lut[k]) || !(lut[k] > 0.f))
+            return qmri_fail(QMRI_EINVAL, "%s: lut(%lld, %d) = %g: T1 and T2 must be finite and > 0", fn, (long long)(k % K + 1), (int)(k / K + 1), lut[k]);
+    QCHECK(w.pulse.ensure(T * sizeof(float4)));
+    QCHECK(w.tr.ensure(T * sizeof(float)));
+    QCHECK(w.lut.ensure((size_t)K * 2 * sizeof(float)));
+    QCUDA(cudaMemcpyAsync(w.pulse.p, pulse.data(), T * sizeof(float4), cudaMemcpyHostToDevice, w.ctx->stream));
+    QCUDA(cudaMemcpyAsync(w.tr.p, tr.data(), T * sizeof(float), cudaMemcpyHostToDevice, w.ctx->stream));
+    QCUDA(cudaMemcpyAsync(w.lut.p, lut, (size_t)K * 2 * sizeof(float), cudaMemcpyHostToDevice, w.ctx->stream));
+    w.p.T = T;
+    w.p.pulse = w.pulse.as<float4>();
+    w.p.tr = w.tr.as<float>();
+    w.p.lut = w.lut.as<float>();
+    w.p.K = K;
+    w.p.te = seq->te;
+    w.p.inversion = seq->inversion;
+    w.p.ti = seq->inversion ? seq->ti : 0.0;
+    return QMRI_OK;
+}
+
+extern "C" int qmri_fisp_signals(qmri_ctx* ctx, const qmri_fisp_seq* seq, const float* lut, int64_t K, float* sig) {
+    if (!ctx || !sig) return qmri_fail(QMRI_EINVAL, "qmri_fisp_signals: null argument");
+    DevSetter ds(ctx->device);
+    FispCall w(ctx);
+    QCHECK(fisp_begin(w, seq, lut, K, "qmri_fisp_signals"));
+    const int T = w.p.T;
+    const int64_t chunk = std::min(K, FISP_CHUNK);
+    QCHECK(w.out.ensure((size_t)T * chunk * sizeof(float)));
+    for (int64_t a0 = 0; a0 < K; a0 += chunk) {
+        const int64_t n = std::min(chunk, K - a0);
+        FispParams p = w.p;
+        p.a0 = a0; p.a1 = a0 + n;
+        p.sig = w.out.as<float>(); p.ld = n;
+        QCHECK(fisp_launch_signals(ctx, p));
+        // device [T][n] -> columns a0 .. a0+n-1 of the K x T column-major host array
+        QCUDA(cudaMemcpy2DAsync(sig + a0, (size_t)K * sizeof(float), p.sig, (size_t)n * sizeof(float), (size_t)n * sizeof(float), T,
+                                cudaMemcpyDeviceToHost, ctx->stream));
+        QCUDA(cudaStreamSynchronize(ctx->stream));  // the chunk buffer is reused
+    }
+    return QMRI_OK;
+}
+
+extern "C" int qmri_fisp_gram(qmri_ctx* ctx, const qmri_fisp_seq* seq, const float* lut, int64_t K, double* G) {
+    if (!ctx || !G) return qmri_fail(QMRI_EINVAL, "qmri_fisp_gram: null argument");
+    DevSetter ds(ctx->device);
+    FispCall w(ctx);
+    QCHECK(fisp_begin(w, seq, lut, K, "qmri_fisp_gram"));
+    const int T = w.p.T, parts = fisp_gram_parts(T);
+    const int64_t chunk = std::min(K, FISP_CHUNK);
+    QCHECK(w.out.ensure((size_t)T * chunk * sizeof(float)));
+    QCHECK(w.part.ensure((size_t)parts * T * T * sizeof(double)));
+    QCHECK(w.G.ensure((size_t)T * T * sizeof(double)));
+    QCUDA(cudaMemsetAsync(w.part.p, 0, (size_t)parts * T * T * sizeof(double), ctx->stream));
+    for (int64_t a0 = 0; a0 < K; a0 += chunk) {  // stream order: each chunk's products are added after the previous chunk's
+        const int64_t n = std::min(chunk, K - a0);
+        FispParams p = w.p;
+        p.a0 = a0; p.a1 = a0 + n;
+        p.sig = w.out.as<float>(); p.ld = n;
+        QCHECK(fisp_launch_signals(ctx, p));
+        QCHECK(fisp_launch_gram_accumulate(ctx, p.sig, n, n, T, w.part.as<double>(), parts));
+    }
+    QCHECK(fisp_launch_gram_reduce(ctx, w.part.as<double>(), parts, T, w.G.as<double>()));
+    QCUDA(cudaMemcpyAsync(G, w.G.p, (size_t)T * T * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    QCUDA(cudaStreamSynchronize(ctx->stream));
+    return QMRI_OK;
+}
+
+extern "C" int qmri_fisp_compress(qmri_ctx* ctx, const qmri_fisp_seq* seq, const float* lut, int64_t K, const double* V, int C,
+                                  int64_t atom_begin, int64_t atom_end, float* D, float* normD) {
+    if (!ctx || !V || !D || !normD) return qmri_fail(QMRI_EINVAL, "qmri_fisp_compress: null argument");
+    DevSetter ds(ctx->device);
+    FispCall w(ctx);
+    QCHECK(fisp_begin(w, seq, lut, K, "qmri_fisp_compress"));
+    const int T = w.p.T;
+    if (C < 1 || C > FISP_MAX_C || C > T) return qmri_fail(QMRI_EINVAL, "qmri_fisp_compress: C = %d outside [1, min(T, %d)]", C, FISP_MAX_C);
+    if (atom_begin < 0 || atom_end > K || atom_begin >= atom_end)
+        return qmri_fail(QMRI_EINVAL, "qmri_fisp_compress: atom range [%lld, %lld) is empty or outside [0, %lld)", (long long)atom_begin,
+                         (long long)atom_end, (long long)K);
+    std::vector<float> Vt((size_t)T * C);  // pulse-major: lane c of the simulating warp reads V(i, c)
+    for (int i = 0; i < T; ++i)
+        for (int c = 0; c < C; ++c) {
+            const double v = V[(size_t)c * T + i];
+            if (!std::isfinite(v)) return qmri_fail(QMRI_EINVAL, "qmri_fisp_compress: V(%d, %d) is not finite", i + 1, c + 1);
+            Vt[(size_t)i * C + c] = (float)v;
+        }
+    const int64_t n = atom_end - atom_begin;
+    QCHECK(w.V.ensure(Vt.size() * sizeof(float)));
+    QCHECK(w.out.ensure((size_t)n * C * sizeof(float)));
+    QCHECK(w.aux.ensure((size_t)n * sizeof(float)));
+    QCUDA(cudaMemcpyAsync(w.V.p, Vt.data(), Vt.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+    FispParams p = w.p;
+    p.a0 = atom_begin; p.a1 = atom_end;
+    p.V = w.V.as<float>(); p.C = C;
+    p.D = w.out.as<float>(); p.normD = w.aux.as<float>();
+    QCHECK(fisp_launch_compress(ctx, p));
+    QCUDA(cudaMemcpyAsync(D, p.D, (size_t)n * C * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    QCUDA(cudaMemcpyAsync(normD, p.normD, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     QCUDA(cudaStreamSynchronize(ctx->stream));
     return QMRI_OK;
 }

@@ -368,6 +368,52 @@ extern "C" void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* 
         plhs[3] = mxCreateNumericMatrix((mwSize)npix, 1, mxINT32_CLASS, mxREAL);
         check(qmri_match(dd, x.p, x.dtype, npix, (float*)mxGetData(plhs[0]), (float*)pd.p, (float*)mxGetData(plhs[2]), (int32_t*)mxGetData(plhs[3])));
         plhs[1] = pd.finish();
+    } else if (cmd == "fisp_signals" || cmd == "fisp_gram" || cmd == "fisp_compress") {
+        // fisp_signals  (lut single K x 2, seq)                     -> sig single K x T
+        // fisp_gram     (lut, seq)                                  -> G double T x T
+        // fisp_compress (lut, seq, V double T x C [, a0, a1])       -> [D single (a1-a0) x C, normD single (a1-a0) x 1]
+        // seq: struct with flip_deg, tr (T doubles), te, ti ([] = no inversion); a0, a1: 0-based atom range [a0, a1)
+        need(3);
+        const mxArray* lut = prhs[1];
+        const mxArray* s = prhs[2];
+        if (!mxIsSingle(lut) || mxIsComplex(lut) || dim_of(lut, 1) != 2) mexErrMsgIdAndTxt("qmri:type", "lut must be real single K x 2 (T1, T2)");
+        const mxArray* flip = mxGetField(s, 0, "flip_deg");
+        const mxArray* tr = mxGetField(s, 0, "tr");
+        const mxArray* te = mxGetField(s, 0, "te");
+        const mxArray* ti = mxGetField(s, 0, "ti");
+        if (!flip || !tr || !te) mexErrMsgIdAndTxt("qmri:param", "seq.flip_deg, seq.tr and seq.te are required");
+        if (!mxIsDouble(flip) || !mxIsDouble(tr) || mxIsComplex(flip) || mxIsComplex(tr))
+            mexErrMsgIdAndTxt("qmri:type", "seq.flip_deg and seq.tr must be real double");
+        if (mxGetNumberOfElements(flip) != mxGetNumberOfElements(tr)) mexErrMsgIdAndTxt("qmri:param", "seq.flip_deg and seq.tr differ in length");
+        qmri_fisp_seq q;
+        memset(&q, 0, sizeof(q));
+        q.T = (int)mxGetNumberOfElements(flip);
+        q.flip_deg = (const double*)mxGetData(flip);
+        q.tr = (const double*)mxGetData(tr);
+        q.te = mxGetScalar(te);
+        q.inversion = ti && mxGetNumberOfElements(ti) > 0;
+        q.ti = q.inversion ? mxGetScalar(ti) : 0.0;
+        const int64_t K = (int64_t)dim_of(lut, 0);
+        const float* L = (const float*)mxGetData(lut);
+        if (cmd == "fisp_signals") {
+            plhs[0] = mxCreateNumericMatrix((mwSize)K, (mwSize)q.T, mxSINGLE_CLASS, mxREAL);
+            check(qmri_fisp_signals(ctx(), &q, L, K, (float*)mxGetData(plhs[0])));
+        } else if (cmd == "fisp_gram") {
+            plhs[0] = mxCreateNumericMatrix((mwSize)q.T, (mwSize)q.T, mxDOUBLE_CLASS, mxREAL);
+            check(qmri_fisp_gram(ctx(), &q, L, K, (double*)mxGetData(plhs[0])));
+        } else {
+            need(4);
+            const mxArray* V = prhs[3];
+            if (!mxIsDouble(V) || mxIsComplex(V)) mexErrMsgIdAndTxt("qmri:type", "V must be real double T x C");
+            const int64_t a0 = nrhs > 5 ? (int64_t)mxGetScalar(prhs[4]) : 0, a1 = nrhs > 5 ? (int64_t)mxGetScalar(prhs[5]) : K;
+            if (dim_of(V, 0) != q.T) mexErrMsgIdAndTxt("qmri:param", "V must have T = %d rows", q.T);
+            const int C = dim_of(V, 1);
+            const mwSize n = a1 > a0 ? (mwSize)(a1 - a0) : 0;
+            plhs[0] = mxCreateNumericMatrix(n, (mwSize)C, mxSINGLE_CLASS, mxREAL);
+            plhs[1] = mxCreateNumericMatrix(n, 1, mxSINGLE_CLASS, mxREAL);
+            check(qmri_fisp_compress(ctx(), &q, L, K, (const double*)mxGetData(V), C, a0, a1, (float*)mxGetData(plhs[0]),
+                                     (float*)mxGetData(plhs[1])));
+        }
     } else if (cmd == "shutdown") {
         shutdown();
     } else {

@@ -43,6 +43,12 @@ class AdmmParams(C.Structure):
                 ("fn_space", C.c_int)]
 
 
+class FispSeq(C.Structure):
+    """qmri_fisp_seq: a FISP schedule (the arrays are borrowed for the duration of a call)."""
+    _fields_ = [("T", C.c_int), ("flip_deg", C.c_void_p), ("tr", C.c_void_p), ("te", C.c_double), ("inversion", C.c_int),
+                ("ti", C.c_double)]
+
+
 # name -> (restype, argtypes); every symbol declared in include/qmri.h
 _vp, _i, _i64, _d = C.c_void_p, C.c_int, C.c_int64, C.c_double
 _pp = C.POINTER(C.c_void_p)
@@ -96,6 +102,9 @@ SIGNATURES = {
     "qmri_foreground_mask": (_i, [_vp, _vp, _i, _i, _i, _d, _vp]),
     "qmri_lrtv": (_i, [_vp, _vp, _i, C.POINTER(LrtvParams), _vp, _i, C.POINTER(C.c_int), C.POINTER(C.c_double)]),
     "qmri_recon_metrics": (_i, [_vp, _i, _i, _i, _vp, _i, _vp, _i, _vp, _vp, _i, _vp, _i, _vp]),
+    "qmri_fisp_signals": (_i, [_vp, C.POINTER(FispSeq), _vp, _i64, _vp]),
+    "qmri_fisp_gram": (_i, [_vp, C.POINTER(FispSeq), _vp, _i64, _vp]),
+    "qmri_fisp_compress": (_i, [_vp, C.POINTER(FispSeq), _vp, _i64, _vp, _i, _i64, _i64, _vp, _vp]),
 }
 
 _lib = None
